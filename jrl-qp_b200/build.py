@@ -5,6 +5,7 @@
 
 The .so files are git-ignored but travel to the GPU box with the gpurun snapshot.
 """
+import concurrent.futures
 import os
 import subprocess
 import sys
@@ -56,30 +57,35 @@ def _includes(path, seen=None):
     return seen
 
 
-def build_cuda(force=False, verbose=False):
-    """One object per .cu (recompiled only when it or a header it includes changed), then one link."""
-    os.makedirs(OUT, exist_ok=True)
-    target = os.path.join(OUT, "libjrlqp_b200.so")
+def build_cuda(force=False, verbose=False, defines=(), out_dir=None):
+    """One object per .cu (recompiled only when it or a header it includes changed), then one link. The objects compile
+    in parallel. defines: extra -D flags (e.g. ["JRLQP_TEST_FALLBACKS"]) for a variant of the library, which then
+    belongs in its own out_dir (default _build)."""
+    out = out_dir or OUT
+    os.makedirs(out, exist_ok=True)
+    target = os.path.join(out, "libjrlqp_b200.so")
+    flags = [f for f in NVCC_FLAGS if f != "-shared"] + ["-D" + d for d in defines]
     srcs = _listdir(CSRC, (".cu",))
-    objs = []
-    logs = []
-    relink = force or not os.path.exists(target)
-    for src in srcs:
-        obj = os.path.join(OUT, os.path.basename(src)[:-3] + ".o")
-        objs.append(obj)
-        if force or _newer(obj, sorted(_includes(src))):
-            cmd = [NVCC] + [f for f in NVCC_FLAGS if f != "-shared"] + ["-c", src, "-o", obj]
-            if verbose:
-                print(" ".join(cmd), file=sys.stderr)
-            res = subprocess.run(cmd, capture_output=True, text=True)
-            logs.append(res.stdout + res.stderr)
-            with open(os.path.join(OUT, os.path.basename(src)[:-3] + ".ptxas.log"), "w") as fh:
-                fh.write(res.stdout + res.stderr)
-            if res.returncode != 0:
-                sys.stderr.write(res.stdout + res.stderr)
-                raise RuntimeError("nvcc failed on " + src)
-            relink = True
-    if relink or _newer(target, objs):
+    objs = [os.path.join(out, os.path.basename(src)[:-3] + ".o") for src in srcs]
+    stale = [(src, obj) for src, obj in zip(srcs, objs) if force or _newer(obj, sorted(_includes(src)))]
+
+    def compile_one(job):
+        src, obj = job
+        cmd = [NVCC] + flags + ["-c", src, "-o", obj]
+        if verbose:
+            print(" ".join(cmd), file=sys.stderr)
+        res = subprocess.run(cmd, capture_output=True, text=True)
+        with open(obj[:-2] + ".ptxas.log", "w") as fh:
+            fh.write(res.stdout + res.stderr)
+        return src, res
+
+    with concurrent.futures.ThreadPoolExecutor(max(1, min(len(stale), os.cpu_count() or 1))) as pool:
+        results = list(pool.map(compile_one, stale))
+    for src, res in results:
+        if res.returncode != 0:
+            sys.stderr.write(res.stdout + res.stderr)
+            raise RuntimeError("nvcc failed on " + src)
+    if stale or force or _newer(target, objs):
         cmd = [NVCC, "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-Xcompiler", "-fPIC"] + objs + ["-o", target]
         if verbose:
             print(" ".join(cmd), file=sys.stderr)

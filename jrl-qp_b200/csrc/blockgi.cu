@@ -458,3 +458,12 @@ extern "C" int jrlqp_blockgi_test_sequence(int32_t device, int32_t n, int32_t nr
   cudaFree(d_rec);
   return rc;
 }
+
+#ifdef JRLQP_TEST_FALLBACKS
+// test build only: this unit's fallback counters and decline flag (test_fallbacks.cuh), read and set through capi.cu
+namespace jrlqp
+{
+int fb_collect_blockgi(unsigned long long * out) { return fb_collect(out); }
+int fb_set_decline_blockgi(int on) { return fb_set_decline(on); }
+} // namespace jrlqp
+#endif

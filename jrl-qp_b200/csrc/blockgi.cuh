@@ -748,6 +748,7 @@ struct BlockGi
         if(!done)
         {
           // an unproven quotient (rare): one link at a time, true divisions
+          JRLQP_FB_HIT_IF(lane == 0, FB_R_SOLVE);
           double wj = w0, rv = 0.0;
           const double dg = Rg[colR(k0 + lc) + k0 + lc];
 #pragma unroll 1

@@ -1412,3 +1412,34 @@ int jrlqp_solve_sequence_host(jrlqp_solver * s, const jrlqp_problem * pb, const 
 }
 
 } // extern "C"
+
+#ifdef JRLQP_TEST_FALLBACKS
+// Test build only (test_fallbacks.cuh): per-site counts of the fallbacks taken, and the flag that makes every proof decline.
+// counts (HOST, 3 x FB_NSITES): the sites reached from this unit (dense and large kernels), from structured.cu (structured
+// LLT and solves) and from blockgi.cu (BlockGI), in that order; the counters are cleared. Device 0.
+namespace jrlqp
+{
+int fb_collect_structured(unsigned long long * out);
+int fb_collect_blockgi(unsigned long long * out);
+int fb_set_decline_structured(int on);
+int fb_set_decline_blockgi(int on);
+} // namespace jrlqp
+
+extern "C" int jrlqp_test_fallback_counts(uint64_t * counts)
+{
+  unsigned long long * c = reinterpret_cast<unsigned long long *>(counts);
+  for(int s = 0; s < 3 * jrlqp::FB_NSITES; ++s) c[s] = 0;
+  int rc = jrlqp::fb_collect(c);
+  if(rc == 0) rc = jrlqp::fb_collect_structured(c + jrlqp::FB_NSITES);
+  if(rc == 0) rc = jrlqp::fb_collect_blockgi(c + 2 * jrlqp::FB_NSITES);
+  return rc;
+}
+
+extern "C" int jrlqp_test_fallback_decline_all(int32_t on)
+{
+  int rc = jrlqp::fb_set_decline(on);
+  if(rc == 0) rc = jrlqp::fb_set_decline_structured(on);
+  if(rc == 0) rc = jrlqp::fb_set_decline_blockgi(on);
+  return rc;
+}
+#endif

@@ -504,6 +504,7 @@ struct GiLarge
               bool ok;
               double cand = div_rcp(w, ld, ri, ok);
               if(!ok && lane == jj) cand = w / ld; // only the lane whose entry is final matters
+              JRLQP_FB_HIT_IF(!ok && lane == jj, FB_LARGE_INIT);
               const double yk = __shfl_sync(JRLQP_FULL, cand, jj);
               if(lane == jj)
                 w = yk;
@@ -519,6 +520,7 @@ struct GiLarge
               bool ok;
               double cand = div_rcp(w, ld, ri, ok);
               if(!ok && lane == jj) cand = w / ld; // only the lane whose entry is final matters
+              JRLQP_FB_HIT_IF(!ok && lane == jj, FB_LARGE_INIT);
               const double xk = __shfl_sync(JRLQP_FULL, cand, jj);
               if(lane == jj)
                 w = xk;

@@ -468,3 +468,12 @@ int jrlqp_structured_solve_host(jrlqp_structured * s,
 }
 
 } // extern "C"
+
+#ifdef JRLQP_TEST_FALLBACKS
+// test build only: this unit's fallback counters and decline flag (test_fallbacks.cuh), read and set through capi.cu
+namespace jrlqp
+{
+int fb_collect_structured(unsigned long long * out) { return fb_collect(out); }
+int fb_set_decline_structured(int on) { return fb_set_decline(on); }
+} // namespace jrlqp
+#endif

@@ -251,7 +251,11 @@ struct TriWarp
       }
       const double w0 = wr;
       bool fast = klo == 0 && khi == NB;
-      if(fast) fast = block_solve_fast<NB, TR>(Ls, dgp + slot * 16, wr, xs);
+      if(fast)
+      {
+        fast = block_solve_fast<NB, TR>(Ls, dgp + slot * 16, wr, xs);
+        JRLQP_FB_HIT_IF(!fast && lane == 0, FB_BLOCK_SOLVE);
+      }
       if(!fast)
       {
         wr = block_solve_exact<NB, TR>(Ls, w0, klo, khi);

@@ -1,10 +1,9 @@
 #!/usr/bin/env python
-"""Development aid: build a variant of libjrlqp_b200.so with extra -D flags on capi.cu (the dense / large kernels; another
-source with VARIANT_SRC=blockgi), re-using the other objects:
-python scripts/build_variant.py <name> -DJRLQP_CH2=28 ...  ->  _build/libjrlqp_b200_<name>.so
-Select it at run time with JRLQP_B200_LIB=<path>."""
+"""Development aid: build a variant of libjrlqp_b200.so with extra -D flags on every source, in its own directory:
+python scripts/build_variant.py <name> -DJRLQP_CH2=28 ...  ->  _build/variants/<name>/libjrlqp_b200.so, copied to
+_build/libjrlqp_b200_<name>.so (the name scripts/ab_variants.py looks for). Select it at run time with JRLQP_B200_LIB=<path>."""
 import os
-import subprocess
+import shutil
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -15,24 +14,17 @@ from jrl_qp_b200 import build as B  # noqa: E402
 
 def main():
     name, flags = sys.argv[1], sys.argv[2:]
-    B.build_cuda()
-    stem = os.environ.get("VARIANT_SRC", "capi")
-    obj = os.path.join(B.OUT, f"{stem}_{name}.o")
-    cmd = [B.NVCC] + [f for f in B.NVCC_FLAGS if f != "-shared"] + flags + ["-c", os.path.join(B.CSRC, stem + ".cu"), "-o", obj]
-    res = subprocess.run(cmd, capture_output=True, text=True)
-    log = res.stdout + res.stderr
-    open(os.path.join(B.OUT, f"{stem}_{name}.ptxas.log"), "w").write(log)
-    if res.returncode != 0:
-        sys.stderr.write(log)
-        sys.exit(1)
+    bad = [f for f in flags if not f.startswith("-D")]
+    if bad:
+        sys.exit(f"only -D flags are supported: {bad}")
+    lib = B.build_cuda(defines=[f[2:] for f in flags], out_dir=os.path.join(B.OUT, "variants", name))
+    log = open(os.path.join(os.path.dirname(lib), "capi.ptxas.log")).read()
     lines = log.splitlines()
     for i, ln in enumerate(lines):
         if "gi_dense_cta_kernelILi" in ln and "Compiling" in ln and "ELb0ELb0" in ln:
             print(ln.split("'")[1][:60], "|", lines[i + 2].strip(), "|", lines[i + 3].strip())
-    bases = [os.path.basename(src)[:-3] for src in B._listdir(B.CSRC, (".cu",))]
-    others = [os.path.join(B.OUT, b + ".o") for b in bases if b != stem]
     out = os.path.join(B.OUT, f"libjrlqp_b200_{name}.so")
-    subprocess.run([B.NVCC, "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-Xcompiler", "-fPIC", obj] + others + ["-o", out], check=True)
+    shutil.copyfile(lib, out)
     print(out)
 
 
