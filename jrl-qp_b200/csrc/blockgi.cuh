@@ -1227,11 +1227,9 @@ struct BlockGi
   }
 };
 
-#ifndef JRLQP_BG_MINB
-#  define JRLQP_BG_MINB 4 // resident CTAs per SM the kernel is compiled for (register cap 65536 / (128 MINB); measured: profiles/r4d_*)
-#endif
+// compiled for 4 resident CTAs per SM (register cap 65536 / (128 * 4); measured: profiles/r4d_*)
 template<int ME>
-__global__ void __launch_bounds__(128, JRLQP_BG_MINB) blockgi_kernel(const BlockGiParams P)
+__global__ void __launch_bounds__(128, 4) blockgi_kernel(const BlockGiParams P)
 {
   extern __shared__ __align__(16) double sm[];
   __shared__ long long next;

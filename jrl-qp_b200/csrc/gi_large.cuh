@@ -28,22 +28,7 @@
 namespace jrlqp
 {
 
-#ifndef JRLQP_LARGE_D_PREFETCH
-#  define JRLQP_LARGE_D_PREFETCH 0 // d = J^T n+: L2 prefetch distance down a thread's own column, in doubles. Measured: 128 -> -1 %, 256 -> -3 % on config C (profiles/r5k_*): off
-#endif
-#ifndef JRLQP_LARGE_D_UNROLL
-#  define JRLQP_LARGE_D_UNROLL 4 // d = J^T n+: iterations (32 bytes of a thread's column each) in flight; 2 -> 4: config C cold +3.9 % (profiles/r5v_ab.txt), no spill
-#endif
-#ifndef JRLQP_WARMB_FAST
-#  define JRLQP_WARMB_FAST 1 // warm start, B = L^-1 N: entries of L loaded one group of rows ahead, quotients from the stored reciprocals (proven)
-#endif
-#ifndef JRLQP_RING_STAGES
-#  define JRLQP_RING_STAGES 3
-#endif
-#ifndef JRLQP_RING_EVICT_FIRST
-#  define JRLQP_RING_EVICT_FIRST 0 // the bulk copies of the column ring carry an L2 evict_first policy (J streams, the shared C should stay)
-#endif
-constexpr int kRingStages = JRLQP_RING_STAGES; // stages of the TMA-fed column ring (see GiLarge::ring_*)
+constexpr int kRingStages = 3; // stages of the TMA-fed column ring (see GiLarge::ring_*)
 
 // Shared-memory carve-up, computed identically on the host (size) and on the device (pointers).
 struct LargeSmem
@@ -212,18 +197,9 @@ struct GiLarge
     const unsigned bytes = (unsigned)(nc * ldl * 8);
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); // earlier generic reads of this stage are done (block barrier)
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-#if JRLQP_RING_EVICT_FIRST
-    unsigned long long pol;
-    asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(
-                   saddr(ring + (long long)stage * rcols * ldl)),
-                 "l"(Jc + (long long)c0 * ldl), "r"(bytes), "r"(bar), "l"(pol)
-                 : "memory");
-#else
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(saddr(ring + (long long)stage * rcols * ldl)),
                  "l"(Jc + (long long)c0 * ldl), "r"(bytes), "r"(bar)
                  : "memory");
-#endif
   }
   __device__ __forceinline__ void ring_wait(const int stage)
   {
@@ -754,7 +730,7 @@ struct GiLarge
       const double blc = act ? bl[c] : 0.0, buc = act ? bu[c] : 0.0;
       // C shared by the batch: scan its transposed copy (made once per call, coalesced across the constraints);
       // lanes whose constraint is active issue no memory request
-      const double cx = P.ct != nullptr ? dot4_col<CH, JRLQP_CT_EVICT_LAST != 0>(P.ct + ct_offset(min(c, mc - 1), n), xs, n, act)
+      const double cx = P.ct != nullptr ? dot4_col<CH, true>(P.ct + ct_offset(min(c, mc - 1), n), xs, n, act)
                                         : (cvec ? dot4_row<true, CH>(ci, xs, n, act) : dot4_row<false, CH>(ci, xs, n, act));
       if(act)
       {
@@ -854,24 +830,18 @@ struct GiLarge
     }
     if(general)
     {
-      // d, thread = column j of the column-major J: 32-byte vector loads down the column
-      constexpr int DU = JRLQP_LARGE_D_UNROLL;
+      // d, thread = column j of the column-major J: 32-byte vector loads down the column, DU of them (iterations) in flight;
+      // 2 -> 4: config C cold +3.9 % (profiles/r5v_ab.txt), no spill. An L2 prefetch down the column lost 1 % (distance 128) and
+      // 3 % (256) on config C (profiles/r5k_*).
+      constexpr int DU = 4;
       for(int j = tid; j < n; j += T)
       {
         const double * Jj = Jc + (long long)j * ldl;
         double a0 = 0, a1 = 0, a2 = 0, a3 = 0;
         int i = 0;
-#if JRLQP_LARGE_D_PREFETCH
-        // every thread walks its own column (3 KB at n = 387) with two 32-byte loads in flight: pull the lines ahead into L2
-        // (the 296 workspaces of 1.2 MB do not fit L2: without the hint every line is an HBM round trip on the dependent path)
-        for(int o = 0; o < JRLQP_LARGE_D_PREFETCH && o < n; o += 16) asm volatile("prefetch.global.L2 [%0];" ::"l"(Jj + o));
-#endif
 #pragma unroll DU
         for(; i + 3 < n; i += 4)
         {
-#if JRLQP_LARGE_D_PREFETCH
-          if((i & 15) == 0 && i + JRLQP_LARGE_D_PREFETCH < n) asm volatile("prefetch.global.L2 [%0];" ::"l"(Jj + i + JRLQP_LARGE_D_PREFETCH));
-#endif
           const double2 p0 = *reinterpret_cast<const double2 *>(Jj + i);
           const double2 p1 = *reinterpret_cast<const double2 *>(Jj + i + 2);
           a0 = fma(p0.x, cv[i], a0);

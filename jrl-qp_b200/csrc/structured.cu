@@ -13,10 +13,6 @@
 
 using namespace jrlqp;
 
-#ifndef JRLQP_STRUCT_DEFAULT_SMALL
-#  define JRLQP_STRUCT_DEFAULT_SMALL 3 // automatic mode on an eligible structure: 2 = small tiles (plain loads), 3 = small tiles + TMA
-#endif
-
 namespace jrlqp
 {
 void count_launch(); // capi.cu: feeds jrlqp_launch_count()
@@ -304,7 +300,8 @@ int jrlqp_structured_llt_device(jrlqp_structured * s, double * data, int64_t str
   p.ok = ok;
   // small uniform tiles: two instances per warp, tiles in registers (structured_small.cuh); needs 16-byte aligned instances
   const bool aligned = (reinterpret_cast<uintptr_t>(data) % 16) == 0 && (stride % 2) == 0;
-  const int mode = s->kernel_mode == 0 ? (s->small_nb && aligned ? JRLQP_STRUCT_DEFAULT_SMALL : 1) : s->kernel_mode;
+  constexpr int kDefaultSmall = 3; // automatic mode on an eligible structure: 2 = small tiles (plain loads), 3 = small tiles + TMA
+  const int mode = s->kernel_mode == 0 ? (s->small_nb && aligned ? kDefaultSmall : 1) : s->kernel_mode;
   if(mode >= 2 && s->small_nb && aligned)
   {
     const bool tma = mode == 3;

@@ -1,7 +1,8 @@
 #!/usr/bin/env python
-"""Development aid: build a variant of libjrlqp_b200.so with extra -D flags on every source, in its own directory:
-python scripts/build_variant.py <name> -DJRLQP_CH2=28 ...  ->  _build/variants/<name>/libjrlqp_b200.so, copied to
-_build/libjrlqp_b200_<name>.so (the name scripts/ab_variants.py looks for). Select it at run time with JRLQP_B200_LIB=<path>."""
+"""Development aid: build a variant of libjrlqp_b200.so, with extra -D flags on every source if any, in its own directory:
+python scripts/build_variant.py <name> [-DJRLQP_TEST_FALLBACKS ...]  ->  _build/variants/<name>/libjrlqp_b200.so, copied to
+_build/libjrlqp_b200_<name>.so (the name scripts/ab_variants.py looks for). Select it at run time with JRLQP_B200_LIB=<path>.
+Tuning values are constants in the sources: to time a different value, build the variant from a branch that changes it."""
 import os
 import shutil
 import sys
