@@ -174,8 +174,10 @@ int jrlqp_solve_batch_host(jrlqp_solver * s, const jrlqp_problem * pb, const jrl
  * reference (FIXED on distinct bounds, a side whose bound is infinite); statuses of the wrong kind
  * (a bound status on a general constraint or vice versa), on which the reference asserts, are ignored.
  * JRLQP_OVERCONSTRAINED_PROBLEM is reported per instance when more than n equalities are given.
- * The shared-memory kernel needs n (n - 1) / 2 more doubles of shared memory than the cold one
- * (n <= ~100); beyond that, select the global-workspace kernel (automatic for n > 128). */
+ * The shared-memory kernel needs n (n - 1) / 2 more doubles of shared memory than the cold one, so it
+ * fits up to n = 115 or so (the limit depends slightly on mc). In automatic mode a warm call whose layout
+ * does not fit runs on the global-workspace kernel (bit-identical results) while cold calls on the same
+ * handle keep the shared-memory kernel; with jrlqp_set_kernel_path(1) it returns JRLQP_ERR_ARG. */
 int jrlqp_solve_batch_warm_device(jrlqp_solver * s, const jrlqp_problem * pb, const jrlqp_result * res, void * stream);
 int jrlqp_solve_batch_warm_host(jrlqp_solver * s, const jrlqp_problem * pb, const jrlqp_result * res);
 

@@ -175,6 +175,7 @@ struct jrlqp_solver
   // large-n kernel (gi_large.cuh): J, L and R live in a per-CTA global-memory workspace
   int path_mode = 0; // 0 automatic (n <= 128: shared-memory kernel), 1 shared-memory kernel, 2 global-workspace kernel
   bool large = false;
+  bool warm_large = false; // automatic mode: the warm layout does not fit in shared memory, warm calls take the large-n kernel
   int lsmem_bytes[2] = {0, 0}, locc[2] = {0, 0}, lregs[2] = {0, 0}; // [cold, warm]
   int lring[2] = {0, 0}; // columns per stage of the TMA column ring of the large-n kernel (0: off)
   int lslab = 0; // rows per slab of J = J Q in the warm large-n kernel (0: off)
@@ -232,6 +233,12 @@ struct jrlqp_solver
   } while(0)
 
 static constexpr int kLargeThreads = 256;
+
+// Kernel family of a call: cold and warm calls on one handle can differ (warm_large)
+static bool large_for(const jrlqp_solver * s, bool warm)
+{
+  return s->large || (warm && s->warm_large);
+}
 
 // Large-n kernel: shared-memory size, residency and the per-CTA global workspace (allocated on first use)
 static int configure_large(jrlqp_solver * s, bool warm)
@@ -535,6 +542,7 @@ int jrlqp_set_kernel_path(jrlqp_solver * s, int32_t mode)
   if(!s || mode < 0 || mode > 2) return JRLQP_ERR_ARG;
   s->path_mode = mode;
   s->wkernel = nullptr;
+  s->warm_large = false;
   cudaSetDevice(s->device);
   return configure_kernel(s);
 }
@@ -608,9 +616,9 @@ static int configure_warm(jrlqp_solver * s);
 // Large-n kernel, G shared by the batch (stride 0): Cholesky and J = L^-T are computed ONCE, by one CTA running the
 // solver's own factorisation code (same bits), and every solver CTA copies them instead of redoing 2/3 n^3 flops per
 // instance (the MultiIK fixtures of config C spend ~100 % of a solve there). Asynchronous on `st`.
-static bool uses_prefactor(const jrlqp_solver * s, const jrlqp_problem * pb)
+static bool uses_prefactor(const jrlqp_solver * s, const jrlqp_problem * pb, bool warm)
 {
-  return s->large && pb->G_stride == 0 && pb->batch >= 2;
+  return large_for(s, warm) && pb->G_stride == 0 && pb->batch >= 2;
 }
 
 static int prefactor(jrlqp_solver * s, const jrlqp_problem * pb, cudaStream_t st)
@@ -640,9 +648,9 @@ static int prefactor(jrlqp_solver * s, const jrlqp_problem * pb, cudaStream_t st
 }
 
 // Large-n kernel, C shared by the batch: one transposed copy per call for the coalesced constraint scan.
-static bool uses_shared_ct(const jrlqp_solver * s, const jrlqp_problem * pb)
+static bool uses_shared_ct(const jrlqp_solver * s, const jrlqp_problem * pb, bool warm)
 {
-  return s->large && s->mc > 0 && pb->C_stride == 0 && pb->batch >= 2 && s->scan_transposed != 0;
+  return large_for(s, warm) && s->mc > 0 && pb->C_stride == 0 && pb->batch >= 2 && s->scan_transposed != 0;
 }
 
 static int prepare_shared_ct(jrlqp_solver * s, const jrlqp_problem * pb, cudaStream_t st)
@@ -688,23 +696,19 @@ static int ensure_ct(jrlqp_solver * s)
 static int launch(jrlqp_solver * s, const jrlqp_problem * pb, const jrlqp_result * res, cudaStream_t st, unsigned long long * counter, bool warm = false, bool force_warm_start = false,
                   bool pre_ready = false)
 {
-  if(s->large)
+  if(warm)
   {
-    int rc = configure_large(s, warm);
+    int rc = configure_warm(s); // (may set warm_large)
     if(rc != JRLQP_OK) return rc;
   }
-  else if(warm)
+  const bool large = large_for(s, warm);
   {
-    int rc = configure_warm(s);
-    if(rc != JRLQP_OK) return rc;
-  }
-  {
-    int rc = ensure_ct(s);
+    int rc = large ? configure_large(s, warm) : ensure_ct(s);
     if(rc != JRLQP_OK) return rc;
   }
   const Layout & lay = warm ? s->wlay : s->lay;
   GiParams p{};
-  if(!s->large && s->mc > 0 && scan_transposed_on(s) && s->d_ct)
+  if(!large && s->mc > 0 && scan_transposed_on(s) && s->d_ct)
   {
     p.ct = s->d_ct;
     p.ct_stride = s->ct_stride;
@@ -777,11 +781,11 @@ static int launch(jrlqp_solver * s, const jrlqp_problem * pb, const jrlqp_result
   p.off_alpha = lay.off_alpha;
   p.fcache = s->d_fcache;
   p.fcache_stride = (long long)s->n * s->n + 2ll * s->n;
-  p.fcache_mode = (warm && !s->large && s->d_fcache != nullptr) ? s->fcache_mode : 0;
-  const int occ = s->large ? s->locc[warm ? 1 : 0] : (warm ? s->wocc : s->occ);
+  p.fcache_mode = (warm && !large && s->d_fcache != nullptr) ? s->fcache_mode : 0;
+  const int occ = large ? s->locc[warm ? 1 : 0] : (warm ? s->wocc : s->occ);
   long long grid = std::min<long long>((long long)occ * s->num_sms, std::max<long long>(pb->batch, 1));
   CK(cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st));
-  if(uses_prefactor(s, pb))
+  if(uses_prefactor(s, pb, warm))
   {
     if(!pre_ready)
     {
@@ -791,7 +795,7 @@ static int launch(jrlqp_solver * s, const jrlqp_problem * pb, const jrlqp_result
     p.pre = s->d_pre;
     p.pre_ok = s->d_pre_ok;
   }
-  if(uses_shared_ct(s, pb))
+  if(uses_shared_ct(s, pb, warm))
   {
     if(!pre_ready)
     {
@@ -801,7 +805,7 @@ static int launch(jrlqp_solver * s, const jrlqp_problem * pb, const jrlqp_result
     p.ct = s->d_cts;
     p.ldct = s->ldcts;
   }
-  if(s->large)
+  if(large)
   {
     p.work = s->d_work[warm ? 1 : 0];
     p.work_stride = s->work_stride[warm ? 1 : 0];
@@ -823,12 +827,20 @@ static int launch(jrlqp_solver * s, const jrlqp_problem * pb, const jrlqp_result
   return JRLQP_OK;
 }
 
+// Shared-memory warm kernel, for handles whose cold calls take the shared-memory kernel. In automatic mode a warm layout
+// that does not fit (n >= ~116: n (n - 1) / 2 more doubles than the cold one) sends the warm calls to the large-n kernel,
+// which computes the same bits; cold calls keep the shared-memory kernel.
 static int configure_warm(jrlqp_solver * s)
 {
-  if(s->wkernel) return JRLQP_OK;
+  if(s->large || s->wkernel || s->warm_large) return JRLQP_OK;
   Layout lay = make_layout(s->n, s->mc, s->nb, s->warps, false, true);
   const int smem = lay.total_doubles * 8;
   KernelFn fn = pick_warm_kernel(s->warps);
+  if(smem > s->max_smem_optin && s->path_mode == 0)
+  {
+    s->warm_large = true;
+    return JRLQP_OK;
+  }
   if(!fn || smem > s->max_smem_optin)
   {
     s->err = "warm start: problem does not fit in shared memory (n too large; the Householder vectors need n (n - 1) / 2 more doubles)";
@@ -987,6 +999,8 @@ static int solve_batch_host_impl(jrlqp_solver * s, const jrlqp_problem * pb, con
   CK(cudaSetDevice(s->device));
   rc = ensure_staging(s, pb, res->L != nullptr);
   if(rc != JRLQP_OK) return rc;
+  if(warm && (rc = configure_warm(s)) != JRLQP_OK) return rc;
+  const bool large = large_for(s, warm);
 
   const long long B = pb->batch;
   const long long n = s->n, mc = s->mc, m = s->m;
@@ -994,7 +1008,7 @@ static int solve_batch_host_impl(jrlqp_solver * s, const jrlqp_problem * pb, con
   // GPU), the kernels read G straight from the caller's PINNED buffer: only the lower triangle crosses PCIe, as
   // SM-initiated reads concurrent with the DMA of the other arrays (measured, profiles/r01u_*: +5 % at n = 50, +9 % at
   // n = 20 over the two-block upload, -5 % at n = 128, which is kernel-bound: automatic mode = n <= 64).
-  const bool zero_copy_G = !s->large && !res->L && pb->G_stride != 0 && (g_zero_copy_G == 1 || (g_zero_copy_G < 0 && s->n <= 64));
+  const bool zero_copy_G = !large && !res->L && pb->G_stride != 0 && (g_zero_copy_G == 1 || (g_zero_copy_G < 0 && s->n <= 64));
   const double * g_dev_ptr_G = nullptr;
   if(zero_copy_G)
   {
@@ -1038,7 +1052,7 @@ static int solve_batch_host_impl(jrlqp_solver * s, const jrlqp_problem * pb, con
       CK(up1(s->d_xl, pb->xl, pb->xl_stride, (int)n, 1, (int)n));
       CK(up1(s->d_xu, pb->xu, pb->xu_stride, (int)n, 1, (int)n));
     }
-    if(s->large && pb->G_stride == 0 && B >= 2)
+    if(large && pb->G_stride == 0 && B >= 2)
     {
       // factor of the shared G, once for the whole call (the chunks below re-use it)
       jrlqp_problem pg{};
@@ -1050,7 +1064,7 @@ static int solve_batch_host_impl(jrlqp_solver * s, const jrlqp_problem * pb, con
       int rcp = prefactor(s, &pg, s->streams[0]);
       if(rcp != JRLQP_OK) return rcp;
     }
-    if(s->large && mc > 0 && pb->C_stride == 0 && B >= 2 && s->scan_transposed != 0)
+    if(large && mc > 0 && pb->C_stride == 0 && B >= 2 && s->scan_transposed != 0)
     {
       jrlqp_problem pc{};
       pc.batch = B;
@@ -1143,7 +1157,7 @@ static int solve_batch_host_impl(jrlqp_solver * s, const jrlqp_problem * pb, con
       dp.as_in = reinterpret_cast<const int8_t *>(das);
       dp.as_stride = pb->as_stride == 0 ? 0 : m;
     }
-    rc = launch(s, &dp, &dr, st, s->d_counters + (c % kMaxChunks), warm, false, /*pre_ready=*/s->large); // shared factor / transposed C prepared above, once for all the chunks
+    rc = launch(s, &dp, &dr, st, s->d_counters + (c % kMaxChunks), warm, false, /*pre_ready=*/large); // shared factor / transposed C prepared above, once for all the chunks
     if(rc != JRLQP_OK) return rc;
     CK(cudaMemcpyAsync(res->x + b0 * n, dr.x, sizeof(double) * cnt * n, cudaMemcpyDeviceToHost, st));
     if(res->u && m) CK(cudaMemcpyAsync(res->u + b0 * m, dr.u, sizeof(double) * cnt * m, cudaMemcpyDeviceToHost, st));
@@ -1216,8 +1230,13 @@ static int sequence_device_impl(jrlqp_solver * s, const jrlqp_problem * pb, cons
     CK(cudaMalloc(&s->d_seq_status, sizeof(int) * (size_t)B));
     s->cap_seq = B;
   }
+  if(seq->warm)
+  {
+    int rc = configure_warm(s);
+    if(rc != JRLQP_OK) return rc;
+  }
   // G is the same at every step: the warm kernels keep the factor of step 0 in HBM and re-read it afterwards (same bits)
-  const bool use_fcache = seq->warm != 0 && !s->large && seq->steps > 1 && !res->L && g_seq_fcache != 0;
+  const bool use_fcache = seq->warm != 0 && !large_for(s, true) && seq->steps > 1 && !res->L && g_seq_fcache != 0;
   if(use_fcache)
   {
     const long long need = B * ((long long)s->n * s->n + 2ll * s->n);

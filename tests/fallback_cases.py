@@ -327,6 +327,8 @@ FAMILY_CASES = _cases([
     ("dense_n100_staged", _dense_cold("n100", 32, stage=1)),
     ("dense_warm_A_wrong", _dense_warm("A", 128, 1, "wrong")),
     ("dense_warm_B_wrong", _dense_warm("B", 256, 1, "wrong")),
+    ("dense_warm_n70_wrong", _dense_warm("n70", 48, 1, "wrong")),    # warm, three warps
+    ("dense_warm_n100_wrong", _dense_warm("n100", 32, 1, "wrong")),  # warm, four warps: branch-free Givens links
     ("large_n160_cold", _dense_cold("n160", 12, path=2)),
     ("large_n160_warm", _dense_warm("n160", 12, 2, "wrong")),
     ("large_n300_cold", _dense_cold("n300", 6, path=2)),
