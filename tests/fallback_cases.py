@@ -35,7 +35,8 @@ def ch_n(n, ne, ni):
 def dense_problem(name, B):
     chs = {"B": P.config_B(), "A": P.config_A(), "D": P.config_D(), "n70": ch_n(70, 5, 150), "n90": ch_n(90, 9, 120),
            "n100": ch_n(100, 10, 110),
-           "weak": P.ProblemCharacteristics(12, 2, 14, 3, 3, 1, 2, True, True), "n160": ch_n(160, 32, 128), "n300": ch_n(300, 60, 240)}
+           "weak": P.ProblemCharacteristics(12, 2, 14, 3, 3, 1, 2, True, True), "n160": ch_n(160, 32, 128), "n300": ch_n(300, 60, 240),
+           "n800": ch_n(800, 80, 720)}
     return P.random_problems(chs[name], B, seed=9000 + chs[name].nVar)
 
 
@@ -118,10 +119,10 @@ def gpu_cold(S, pb, path=0, stage=-1, big_bnd=None, want_L=False):
     return {k: sv.last[k] for k in QP_KEYS + (("L",) if want_L else ())}
 
 
-def gpu_warm(S, pb, as_in, path=0, big_bnd=None):
+def gpu_warm(S, pb, as_in, path=0, big_bnd=None, max_iter=500):
     sv = S.BatchedGoldfarbIdnaniSolver(pb.n, pb.mc, pb.nb > 0, pb.batch)
     sv.set_kernel_path(path)
-    o = S.SolverOptions().warmStart(True)
+    o = S.SolverOptions().warmStart(True).maxIter(max_iter)
     if big_bnd is not None:
         o.bigBnd(big_bnd)
     sv.options(o)
@@ -134,9 +135,9 @@ def oracle_cold(pb, big_bnd=1e100):
     return {k: r[k] for k in QP_KEYS}
 
 
-def oracle_warm(pb, as_in, big_bnd=1e100):
+def oracle_warm(pb, as_in, big_bnd=1e100, max_iter=500):
     r = po.solve_batch(pb.G, pb.a, pb.C, pb.bl, pb.bu, pb.xl, pb.xu, big_bnd=big_bnd, nthreads=_nthreads(), experimental=True,
-                       warm_start=True, as_in=as_in)
+                       warm_start=True, as_in=as_in, max_iter=max_iter)
     return {k: r[k] for k in QP_KEYS}
 
 
@@ -252,7 +253,7 @@ def _dense_cold(name, B, path=0, stage=-1, s=1.0, want_L=True):
     return (lambda S: gpu_cold(S, pb(), path, stage, bb, want_L)), (lambda: oracle_cold(pb(), 1e100 if bb is None else bb))
 
 
-def _dense_warm(name, B, path, guess, s=1.0):
+def _dense_warm(name, B, path, guess, s=1.0, max_iter=500):
     """Warm start from the oracle's cold active set ("exact") or from a wrong guess derived from it."""
     def inputs():
         pb0 = dense_problem(name, B)
@@ -263,12 +264,22 @@ def _dense_warm(name, B, path, guess, s=1.0):
 
     def run(S):
         pb, as_in = inputs()
-        return gpu_warm(S, pb, as_in, path, bb)
+        return gpu_warm(S, pb, as_in, path, bb, max_iter)
 
     def oracle():
         pb, as_in = inputs()
-        return oracle_warm(pb, as_in, 1e100 if bb is None else bb)
+        return oracle_warm(pb, as_in, 1e100 if bb is None else bb, max_iter)
     return run, oracle
+
+
+def _dense_shared(name, B):
+    """G, C and bounds shared by the batch, a per instance: the large kernel factorises G once (prefactor kernel) and
+    every CTA computes x = -G^-1 a from the shared factor in initial_point_blocked."""
+    def sh():
+        pb = dense_problem(name, B)
+        a = pb.a[0] + 0.05 * np.random.default_rng(1).standard_normal(pb.a.shape)
+        return P.ProblemBatch(pb.G[0], a, pb.C[0], pb.bl[0], pb.bu[0], pb.xl[0], pb.xu[0])
+    return (lambda S: gpu_cold(S, sh(), 2)), (lambda: oracle_cold(_replicated(sh())))
 
 
 def _multiik(which, B, warm):
@@ -333,6 +344,10 @@ FAMILY_CASES = _cases([
     ("large_n160_warm", _dense_warm("n160", 12, 2, "wrong")),
     ("large_n300_cold", _dense_cold("n300", 6, path=2)),
     ("large_n300_warm", _dense_warm("n300", 6, 2, "wrong")),
+    ("large_n800_cold", _dense_cold("n800", 3, path=2)),        # four rows per thread, no column ring
+    ("large_n800_warm", _dense_warm("n800", 3, 2, "wrong", max_iter=2000)),  # warm, J = J Q without shared-memory slabs
+                                                                              # (about 670 iterations)
+    ("large_n800_shared", _dense_shared("n800", 3)),            # prefactor of the shared G, initial_point_blocked
     ("multiik_seq_cold", _multiik("sequential", 6, False)),    # G and C shared by the batch
     ("multiik_seq_warm", _multiik("sequential", 6, True)),
     ("multiik_sim_cold", _multiik("simultaneous", 6, False)),

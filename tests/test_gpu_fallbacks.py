@@ -62,6 +62,9 @@ EDGE_SITES = {
     "dyadic_I_large": [(0, 1), (0, 2)],
     "dyadic_sequence": [(0, 3), (0, 4)],
 }
+# sites of the global-workspace kernel at four rows per thread, with every proof declined
+# (initial_point_blocked runs only from the factor of a batch-shared G; a per-instance G takes the serial initial_point)
+LARGE_N_SITES = {"large_n800_cold": [(0, 1)], "large_n800_warm": [(0, 7)], "large_n800_shared": [(0, 6)]}
 # (warm starts of the scaled problems from the unscaled cold active set: oracle parity only — the oracle itself does not
 # keep the relation there)
 RELATION_QP = ["binade_A", "binade_B", "binade_D", "binade_n70", "binade_n300"]
@@ -138,6 +141,15 @@ def test_decline_all_reaches_every_site(variant):
     total = np.sum([np.asarray(c, dtype=np.int64) for c in counts.values()], axis=0)
     missed = [f"{UNITS[u]}:{SITES[s]}" for u, s in ALL_SITES if total[u * NS + s] == 0]
     assert not missed, f"fallback sites never taken with every proof declined: {missed}"
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("name", list(LARGE_N_SITES))
+def test_decline_all_reaches_the_large_kernel_sites_at_n_800(variant, name):
+    _, counts = variant["decline"]
+    c = counts[name]
+    missed = [f"{UNITS[u]}:{SITES[s]}" for u, s in LARGE_N_SITES[name] if c[u * NS + s] == 0]
+    assert not missed, f"{name} does not reach {missed} with every proof declined (counts {_names(c)})"
 
 
 @pytest.mark.gpu

@@ -1,20 +1,25 @@
-"""An extended-precision reference for the warm-start solver, independent of oracle/warm_oracle.cpp.
+"""An extended-precision reference for the solver, independent of the oracles (oracle/gi_oracle.cpp, warm_oracle.cpp).
 
 Whatever path the solver took, its result must be the solution of the equality-constrained QP on the active set it
 reports: K [x; lam] = [-a; b] with K = [[G, -N^T], [N, 0]], N the normals of the active constraints (rows of C or unit
 vectors) and b their active bounds. The warm start reaches that point through its own formulas (x = J1 beta - J2 alpha2,
-u = R^-1 (alpha1 + beta), f = beta . (beta / 2 + alpha1) - |alpha2|^2 / 2), so this checks them against plain linear
-algebra: K is solved in float64 and refined with residuals computed in 200-bit arithmetic (mpmath), which gives the
-solution to float64 accuracy while cond(K) eps << 1. The solver's multipliers are u = -lam on the active entries and
-exactly 0 elsewhere.
+u = R^-1 (alpha1 + beta), f = beta . (beta / 2 + alpha1) - |alpha2|^2 / 2), and the cold solver through a sequence of
+rank-one updates, so this checks them against plain linear algebra: K is solved in float64 and refined with residuals
+that are correctly rounded (each product exact as p + e by Dekker's split, each row summed by math.fsum), which gives
+the solution to float64 accuracy while cond(K) eps << 1. The solver's multipliers are u = -lam on the active entries
+and exactly 0 elsewhere.
 
-This module holds the reference and pins the oracle to it on the CPU; tests/test_gpu_warm_widths.py applies the same
-check to the GPU's warm outputs."""
+This module holds the reference and pins the oracle to it on the CPU; tests/test_gpu_warm_widths.py and
+tests/test_gpu_large_n.py apply the same check to the GPU's outputs."""
+import functools
+import math
 import os
+import time
 
 import mpmath
 import numpy as np
 import pytest
+import scipy.linalg as sla
 
 import pyoracle as po
 from fallback_cases import wrong_guess
@@ -37,13 +42,33 @@ def slot_characteristics(n):
     return P.ProblemCharacteristics(n, ne, ni, min(ni, max(0, n // 4)), 0, min(n // 10, n - ne - min(ni, n // 4)), 0, True, True)
 
 
-def _residual(rows, z, rhs):
-    """rhs - K z, each entry computed in 200-bit arithmetic from the float64 entries, then rounded once."""
-    zm = [mpmath.mpf(float(v)) for v in z]
-    return np.array([float(mpmath.mpf(float(r)) - mpmath.fdot(vals, [zm[j] for j in cols])) for (cols, vals), r in zip(rows, rhs)])
+_SPLIT = 134217729.0  # 2^27 + 1: Dekker's split of a double into two halves of at most 26 significant bits
 
 
-def kkt_reference(G, a, C, bl, bu, xl, xu, act, refinements=3):
+def _two_products(A, z):
+    """p, e with p + e = A * z exactly, elementwise (Dekker's product; numpy never contracts a * b + c into an FMA).
+    Exact while no product over- or underflows, as with the O(1) data of these tests."""
+    def split(v):
+        c = _SPLIT * v
+        hi = c - (c - v)
+        return hi, v - hi
+    p = A * z
+    ah, al = split(A)
+    zh, zl = split(z)
+    return p, ((ah * zh - p) + ah * zl + al * zh) + al * zl
+
+
+def _residual(K, z, rhs):
+    """rhs - K z, each entry correctly rounded: math.fsum of rhs_i and the exact products of row i (its nonzeros)."""
+    p, e = _two_products(K, z[None, :])
+    out = np.empty(K.shape[0])
+    for i, row in enumerate(K):
+        nz = row != 0
+        out[i] = math.fsum(np.concatenate([[rhs[i]], -p[i, nz], -e[i, nz]]).tolist())
+    return out
+
+
+def kkt_reference(G, a, C, bl, bu, xl, xu, act, refinements=3, residual=_residual):
     """x*, u*, f* and cond(K) of one instance (arrays of one instance, layout of solve_batch) on the active set `act`."""
     n = a.shape[0]
     mc = 0 if C is None else C.shape[0]
@@ -61,34 +86,37 @@ def kkt_reference(G, a, C, bl, bu, xl, xu, act, refinements=3):
     q = active.size
     K = np.block([[G, -N.T], [N, np.zeros((q, q))]])
     rhs = np.concatenate([-a, b])
-    rows = []
-    for row in K:
-        cols = np.flatnonzero(row)
-        rows.append((cols, [mpmath.mpf(float(v)) for v in row[cols]]))
-    with mpmath.workprec(200):
-        z = np.linalg.solve(K, rhs)
-        for _ in range(refinements):
-            z = z + np.linalg.solve(K, _residual(rows, z, rhs))
-        xs = z[:n]
-        xm = [mpmath.mpf(float(v)) for v in xs]
-        Gx = [mpmath.fdot([mpmath.mpf(float(v)) for v in G[i]], xm) for i in range(n)]
-        fs = float(mpmath.fdot(xm, Gx) / 2 + mpmath.fdot([mpmath.mpf(float(v)) for v in a], xm))
+    z = np.linalg.solve(K, rhs)
+    for _ in range(refinements):
+        z = z + np.linalg.solve(K, residual(K, z, rhs))
+    xs = z[:n]
+    # f* = x*.(G x*) / 2 + a.x*, with G x* rounded once per row and the rest summed exactly
+    p, e = _two_products(np.concatenate([0.5 * xs, a]), np.concatenate([-_residual(G, xs, np.zeros(n)), xs]))
+    fs = math.fsum(np.concatenate([p, e]).tolist())
     us = np.zeros(act.size)
     us[active] = -z[n:]
-    return xs, us, fs, np.linalg.cond(K)
+    # cond_2(K) from the symmetric [[G, N^T], [N, 0]] = K diag(I, -I), whose |eigenvalues| are the singular values of K: at
+    # n = 1024 the eigenvalues take 0.1 s, the SVD of np.linalg.cond 0.5 s and numpy's own eigvalsh over 1 s
+    ev = np.abs(sla.eigh(np.block([[G, N.T], [N, np.zeros((q, q))]]), eigvals_only=True))
+    return xs, us, fs, ev.max() / ev.min()
+
+
+def _sampled_instances(pb, out, sample, what):
+    """(b, arguments of kkt_reference) of up to `sample` successful instances of `out`, spread over the batch."""
+    ok = np.flatnonzero(out["status"] == 0)
+    assert ok.size > 0, f"{what}: no successful instance to check"
+    for b in ok[np.unique(np.linspace(0, ok.size - 1, min(sample, ok.size)).astype(int))]:
+        G = pb.G[b] if pb.G.ndim == 3 else pb.G
+        C = None if pb.mc == 0 else (pb.C[b] if pb.C.ndim == 3 else pb.C)
+        bl, bu, xl, xu = ((None if v is None else (v[b] if v.ndim == 2 else v)) for v in (pb.bl, pb.bu, pb.xl, pb.xu))
+        yield b, (G, pb.a[b], C, bl, bu, xl, xu, out["active_set"][b])
 
 
 def assert_matches_kkt_reference(pb, out, sample=8, what=""):
     """Up to `sample` successful instances of `out`, spread over the batch, against kkt_reference."""
-    ok = np.flatnonzero(out["status"] == 0)
-    assert ok.size > 0, f"{what}: no successful instance to check"
-    pick = ok[np.unique(np.linspace(0, ok.size - 1, min(sample, ok.size)).astype(int))]
-    for b in pick:
-        G = pb.G[b] if pb.G.ndim == 3 else pb.G
-        C = None if pb.mc == 0 else (pb.C[b] if pb.C.ndim == 3 else pb.C)
-        bl, bu, xl, xu = ((None if v is None else (v[b] if v.ndim == 2 else v)) for v in (pb.bl, pb.bu, pb.xl, pb.xu))
-        act = out["active_set"][b]
-        xs, us, fs, kappa = kkt_reference(G, pb.a[b], C, bl, bu, xl, xu, act)
+    for b, args in _sampled_instances(pb, out, sample, what):
+        act = args[-1]
+        xs, us, fs, kappa = kkt_reference(*args)
         tag = f"{what} instance {b}"
         assert kappa <= KAPPA_MAX, f"{tag}: cond(K) = {kappa:.3g}, the bound would be meaningless"
         tol = TOL_FACTOR * EPS * kappa
@@ -136,23 +164,70 @@ def test_kkt_reference_solves_a_known_problem():
     assert kappa < 10
 
 
+@functools.lru_cache(maxsize=None)
+def _width_case(n):
+    """16 instances of the slot recipe at n, and the oracle's warm starts from the exact and from a wrong guess."""
+    pb = P.random_problems(slot_characteristics(n), 16, seed=n)
+    act = oracle_cold(pb)["active_set"]
+    return pb, act, oracle_warm(pb, act), oracle_warm(pb, wrong_guess(act, pb.mc, seed=n))
+
+
+@functools.lru_cache(maxsize=None)
+def _full_rank_case(n, eq):
+    pb = full_rank_problem(n, n if eq == "all" else n // 2, 8, seed=300 + n)
+    return pb, oracle_warm(pb, oracle_cold(pb)["active_set"])
+
+
 @pytest.mark.parametrize("n", WIDTHS)
 def test_oracle_warm_start_matches_extended_precision_kkt(n):
     """The oracle's warm start from the exact and from a wrong guess, every width of the GPU tests."""
-    pb = P.random_problems(slot_characteristics(n), 16, seed=n)
-    act = oracle_cold(pb)["active_set"]
-    exact = oracle_warm(pb, act)
+    pb, act, exact, wrong = _width_case(n)
     assert (exact["iterations"] == 0).all()
     assert_matches_kkt_reference(pb, exact, what=f"n={n} exact")
-    assert_matches_kkt_reference(pb, oracle_warm(pb, wrong_guess(act, pb.mc, seed=n)), what=f"n={n} wrong")
+    assert_matches_kkt_reference(pb, wrong, what=f"n={n} wrong")
 
 
 @pytest.mark.parametrize("n", [20, 33, 70, 100])
 @pytest.mark.parametrize("eq", ["all", "half"])
 def test_oracle_warm_start_with_n_active_constraints_matches_kkt(n, eq):
     """q = n: N fixes x alone and the multipliers come from the first block row."""
-    pb = full_rank_problem(n, n if eq == "all" else n // 2, 8, seed=300 + n)
-    act = oracle_cold(pb)["active_set"]
-    r = oracle_warm(pb, act)
+    pb, r = _full_rank_case(n, eq)
     assert (r["status"] == 0).all() and (r["n_active"] == n).all()
     assert_matches_kkt_reference(pb, r, what=f"n={n} q=n ({eq} equalities)")
+
+
+def _residual_mpmath(K, z, rhs):
+    """rhs - K z, each entry computed in 200-bit arithmetic from the float64 entries, then rounded once."""
+    with mpmath.workprec(200):
+        zm = [mpmath.mpf(float(v)) for v in z]
+        return np.array([float(mpmath.mpf(float(r)) - mpmath.fdot([mpmath.mpf(float(v)) for v in row[c]], [zm[j] for j in c]))
+                         for row, r in zip(K, rhs) for c in (np.flatnonzero(row),)])
+
+
+@pytest.mark.parametrize("case", [("slot", n) for n in WIDTHS] + [("q=n", n, eq) for n in (20, 33, 70, 100) for eq in ("all", "half")],
+                         ids=lambda c: "-".join(map(str, c)))
+def test_exact_residual_refines_to_the_same_bits_as_200_bit_arithmetic(case):
+    """The correctly rounded residual (Dekker products, math.fsum) and a 200-bit mpmath residual lead the refinement to the
+    same x* and u*, on every instance the tests above check."""
+    if case[0] == "slot":
+        pb, _, exact, wrong = _width_case(case[1])
+        outs = [(pb, exact), (pb, wrong)]
+    else:
+        outs = [_full_rank_case(*case[1:])]
+    for pb, out in outs:
+        for b, args in _sampled_instances(pb, out, 8, str(case)):
+            x1, u1, _, _ = kkt_reference(*args)
+            x2, u2, _, _ = kkt_reference(*args, residual=_residual_mpmath)
+            assert np.array_equal(x1, x2), f"{case} instance {b}: x* differs"
+            assert np.array_equal(u1, u2), f"{case} instance {b}: u* differs"
+
+
+def test_oracle_cold_matches_extended_precision_kkt_at_n_1024():
+    """The cold oracle at the top of the supported range (slot recipe, up to 2000 iterations) against the reference,
+    which stays fast enough there to sample many instances of a batch."""
+    pb = P.random_problems(slot_characteristics(1024), 2, seed=1024)
+    r = po.solve_batch(pb.G, pb.a, pb.C, pb.bl, pb.bu, pb.xl, pb.xu, nthreads=os.cpu_count(), max_iter=2000)
+    assert (r["status"] == 0).all()
+    t0 = time.perf_counter()
+    assert_matches_kkt_reference(pb, r, what="n=1024 cold")
+    print(f"kkt_reference at n = 1024: {(time.perf_counter() - t0) / pb.batch:.2f} s per instance")
