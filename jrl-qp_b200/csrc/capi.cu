@@ -63,18 +63,9 @@ KernelFn pick_kernel(int warps, bool stage)
   }
 }
 
-struct Layout
+DenseSmem make_layout(int n, int mc, int nb, int warps, bool stage, bool warm = false)
 {
-  int ldj, ldcs, npad;
-  int off_R, off_x, off_z, off_d, off_r, off_u, off_cv, off_gc, off_gs, off_gcs, off_ldiag, off_rinv, off_scr, off_C;
-  int off_alist, off_gk, off_iscr, off_stat, off_eq, off_il;
-  int off_V, off_bact, off_hco, off_alpha;
-  int total_doubles;
-};
-
-Layout make_layout(int n, int mc, int nb, int warps, bool stage, bool warm = false)
-{
-  Layout L{};
+  DenseSmem L{};
   L.ldj = n | 1;
   L.ldcs = n | 1;
   L.npad = 32 * warps;
@@ -96,7 +87,7 @@ Layout make_layout(int n, int mc, int nb, int warps, bool stage, bool warm = fal
   L.off_cv = o;
   o += np;
   o += o & 1; // 16-byte alignment of the per-link records of the Givens sweep
-  L.off_gc = L.off_gs = L.off_gcs = o; // (one array of 32-byte records: see GiCta::givens_recurrence)
+  L.off_gcs = o; // (one array of 32-byte records: see GiCta::givens_recurrence)
   o += 4 * np;
   L.off_ldiag = o;
   o += np;
@@ -108,7 +99,6 @@ Layout make_layout(int n, int mc, int nb, int warps, bool stage, bool warm = fal
   o += stage ? mc * L.ldcs : 0;
   L.off_alist = o;
   o += np / 2 + 1;
-  L.off_gk = o; // (unused: the branch taken lives in the records)
   L.off_iscr = o;
   o += 8;
   L.off_stat = o;
@@ -133,6 +123,34 @@ Layout make_layout(int n, int mc, int nb, int warps, bool stage, bool warm = fal
   return L;
 }
 
+// Everything a launch of one kind of call (cold or warm) needs: the kernel, its size and residency, and either the
+// shared-memory layout of the dense kernel or the per-CTA workspace of the global-workspace (large-n) kernel.
+struct LaunchCfg
+{
+  KernelFn fn = nullptr; // null: not configured
+  int threads = 0, smem = 0, occ = 0, regs = 0; // per CTA: threads, dynamic shared-memory bytes; resident CTAs per SM; registers
+  bool large = false; // the global-workspace kernel (gi_large.cuh)
+  // dense kernel
+  bool stage = false; // C staged in shared memory
+  DenseSmem lay{};
+  // large-n kernel
+  int ring_cols = 0; // columns per stage of the TMA column ring (0: off)
+  int slab_rows = 0; // rows per slab of J = J Q, warm kernel (0: off)
+  double * work = nullptr;
+  int * busy = nullptr;
+  int work_slots = 0;
+  long long work_stride = 0;
+};
+
+// What a call asks of launch() besides its problem and result
+struct CallArgs
+{
+  bool warm = false; // the warm-start capable solver
+  bool force_warm_start = false; // honour as_in whatever options().warm_start says (sequences)
+  bool pre_ready = false; // the factor of a shared G and the transposed shared C were prepared earlier on the stream
+  int fcache_mode = 0; // sequence factor cache (gi_params.h: fcache_mode)
+};
+
 } // namespace
 
 namespace jrlqp
@@ -151,43 +169,27 @@ struct jrlqp_solver
   jrlqp_options opt{};
   int warps = 1;
   int stage_mode = -1; // -1 auto
-  bool stage = false;
-  Layout lay{};
-  KernelFn kernel = nullptr;
-  int smem_bytes = 0;
-  int occ = 0;
-  // warm-start (experimental solver) kernel: own shared-memory layout, configured on first use
-  Layout wlay{};
-  KernelFn wkernel = nullptr;
-  int wsmem_bytes = 0;
-  int wocc = 0;
+  int path_mode = 0; // 0 automatic (n <= 128: shared-memory kernel), 1 shared-memory kernel, 2 global-workspace kernel
+  // [cold, warm]: what serves each kind of call. Cold: configured at creation and by set_kernel_path / set_stage_c. Warm
+  // (experimental solver): configured on the first warm call, reset by set_kernel_path.
+  LaunchCfg cfg[2];
+  // [cold, warm]: the global-workspace kernel of each family, configured on first use; its workspace lives as long as the handle
+  LaunchCfg large_cfg[2];
   signed char * d_as = nullptr; // staging of as_in for the host entry point
   // warm-started sequences (jrlqp_solve_sequence_*): scratch for per-step iterations / status and host staging
   double * d_fcache = nullptr; // factor of step 0 of a warm-started sequence (gi_params.h: fcache), re-read by the later steps
   long long fcache_cap = 0; // doubles
-  int fcache_mode = 0; // mode of the next launch (set by sequence_device_impl only)
   int * d_seq_it = nullptr;
   int * d_seq_status = nullptr;
   long long cap_seq = 0;
   double * d_seq = nullptr; // arena: linear terms of all steps + per-step outputs (host entry point)
   long long cap_seq_arena = 0;
   int * d_seq_tot = nullptr; // [2][capacity]: iterations_total, status_worst (host entry point)
-  // large-n kernel (gi_large.cuh): J, L and R live in a per-CTA global-memory workspace
-  int path_mode = 0; // 0 automatic (n <= 128: shared-memory kernel), 1 shared-memory kernel, 2 global-workspace kernel
-  bool large = false;
-  bool warm_large = false; // automatic mode: the warm layout does not fit in shared memory, warm calls take the large-n kernel
-  int lsmem_bytes[2] = {0, 0}, locc[2] = {0, 0}, lregs[2] = {0, 0}; // [cold, warm]
-  int lring[2] = {0, 0}; // columns per stage of the TMA column ring of the large-n kernel (0: off)
-  int lslab = 0; // rows per slab of J = J Q in the warm large-n kernel (0: off)
-  double * d_work[2] = {nullptr, nullptr};
   double * d_cts = nullptr; // transposed copy of a batch-shared C (large-n kernel)
   int ldcts = 0;
   double * d_pre = nullptr; // factor of a batch-shared G (large-n kernel), see gi_params.h
   int * d_pre_ok = nullptr;
   int pre_smem = 0;
-  int * d_busy[2] = {nullptr, nullptr};
-  int work_slots[2] = {0, 0};
-  long long work_stride[2] = {0, 0};
   // capacity (instances) of every staging buffer of the host entry point: 1 for arrays shared by the batch
   long long cap_G = 0, cap_a = 0, cap_C = 0, cap_bl = 0, cap_bu = 0, cap_xl = 0, cap_xu = 0, cap_out = 0, cap_L = 0;
   // transposed copy of C for the coalesced constraint scan of the non-staged shared-memory kernels
@@ -197,7 +199,6 @@ struct jrlqp_solver
   int ct_slots = 0, ldct = 0;
   long long ct_stride = 0;
   int num_sms = 0;
-  int regs = 0;
   int max_smem_optin = 0;
   // device-side scratch
   unsigned long long * d_counters = nullptr; // kMaxChunks counters
@@ -234,17 +235,23 @@ struct jrlqp_solver
 
 static constexpr int kLargeThreads = 256;
 
-// Kernel family of a call: cold and warm calls on one handle can differ (warm_large)
-static bool large_for(const jrlqp_solver * s, bool warm)
+// CTAs of `fn` resident per SM at `threads` threads and `smem` bytes of dynamic shared memory; 0 when that size does not
+// fit (the error of the failed call cleared).
+static int resident_ctas(const jrlqp_solver * s, KernelFn fn, int threads, int smem)
 {
-  return s->large || (warm && s->warm_large);
+  int occ = 0;
+  if(smem > s->max_smem_optin) return 0;
+  if(jrlqp::raise_smem_limit(fn, smem) != cudaSuccess || cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, threads, smem) != cudaSuccess)
+  {
+    cudaGetLastError();
+    return 0;
+  }
+  return occ;
 }
 
-// Large-n kernel: shared-memory size, residency and the per-CTA global workspace (allocated on first use)
-static int configure_large(jrlqp_solver * s, bool warm)
+// Large-n kernel: shared-memory size, residency and the per-CTA global workspace
+static int configure_large(jrlqp_solver * s, bool warm, LaunchCfg & c)
 {
-  const int w = warm ? 1 : 0;
-  if(s->d_work[w]) return JRLQP_OK;
   KernelFn fn = warm ? gi_large_kernel<kLargeThreads, true> : gi_large_kernel<kLargeThreads, false>;
   const LargeSmem lay(s->n, s->m, warm);
   const int smem = lay.total * 8;
@@ -253,9 +260,7 @@ static int configure_large(jrlqp_solver * s, bool warm)
     s->err = "large-n kernel: the vectors do not fit in shared memory";
     return JRLQP_ERR_ARG;
   }
-  CK(jrlqp::raise_smem_limit(fn, smem));
-  int occ = 0;
-  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, kLargeThreads, smem));
+  int occ = resident_ctas(s, fn, kLargeThreads, smem);
   if(occ < 1)
   {
     s->err = "large-n kernel cannot be made resident";
@@ -266,7 +271,7 @@ static int configure_large(jrlqp_solver * s, bool warm)
   // The streaming passes over J (rotation sweep of an add, z = J2 d2) read their columns through a ring of shared-memory stages
   // filled by TMA bulk copies (gi_large.cuh: ring_*), when the rows fit two per thread and the stages cost no residency.
   int smem_total = smem;
-  s->lring[w] = 0;
+  c.ring_cols = 0;
   {
     // Measured (profiles/r5i_*, 32 768 QPs): n = 387 cold 109.4 k -> 132.1 k QP/s (+21 %: 296 workspaces of 1.2 MB do not fit L2, the
     // sweeps wait on HBM); n = 210 cold -3 % (104 MB of workspaces stay in L2 and the stages take 40 KB of L1 away), warm starts
@@ -279,22 +284,18 @@ static int configure_large(jrlqp_solver * s, bool warm)
     if(want && s->n <= 2 * kLargeThreads && rc >= 4)
     {
       const int with_ring = ((lay.total + 1) & ~1) * 8 + (int)jrlqp::large_ring_doubles(s->n, rc) * 8;
-      int occ2 = 0;
-      if(with_ring <= s->max_smem_optin && jrlqp::raise_smem_limit(fn, with_ring) == cudaSuccess
-         && cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ2, fn, kLargeThreads, with_ring) == cudaSuccess && occ2 >= occ)
+      if(resident_ctas(s, fn, kLargeThreads, with_ring) >= occ)
       {
-        s->lring[w] = rc;
+        c.ring_cols = rc;
         smem_total = with_ring;
       }
-      else
-        cudaGetLastError();
     }
   }
+  c.slab_rows = 0;
   if(warm)
   {
     // J = J Q of the warm start on slabs of 16 / 8 rows of J in shared memory (gi_large_warm.inl: warm_JQ_slab), when they cost
     // no residency. JRLQP_LARGE_SLAB=0: off (the thread = row version on the global workspace).
-    s->lslab = 0;
     const char * e = getenv("JRLQP_LARGE_SLAB");
     if(!e || e[0] != '0')
     {
@@ -304,31 +305,45 @@ static int configure_large(jrlqp_solver * s, bool warm)
         const long long bytes = jrlqp::large_slab_doubles(s->n, R) * 8;
         if(bytes > 36 * 1024) continue;
         const int tot = base + (int)bytes;
-        int occ2 = 0;
-        if(tot <= s->max_smem_optin && jrlqp::raise_smem_limit(fn, tot) == cudaSuccess
-           && cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ2, fn, kLargeThreads, tot) == cudaSuccess && occ2 >= occ)
+        if(resident_ctas(s, fn, kLargeThreads, tot) >= occ)
         {
-          s->lslab = R;
+          c.slab_rows = R;
           smem_total = tot;
           break;
         }
-        cudaGetLastError();
       }
     }
   }
   cudaFuncAttributes attr;
   CK(cudaFuncGetAttributes(&attr, fn));
-  s->lregs[w] = attr.numRegs;
-  s->lsmem_bytes[w] = smem_total;
-  s->locc[w] = occ;
-  s->work_stride[w] = large_workspace_doubles(s->n, warm);
-  s->work_slots[w] = slots;
-  CK(cudaMalloc(&s->d_busy[w], sizeof(int) * (size_t)slots));
-  CK(cudaMemset(s->d_busy[w], 0, sizeof(int) * (size_t)slots));
-  CK(cudaMalloc(&s->d_work[w], sizeof(double) * (size_t)s->work_stride[w] * (size_t)slots));
+  c.regs = attr.numRegs;
+  c.threads = kLargeThreads;
+  c.smem = smem_total;
+  c.occ = occ;
+  c.large = true;
+  c.work_stride = large_workspace_doubles(s->n, warm);
+  c.work_slots = slots;
+  CK(cudaMalloc(&c.busy, sizeof(int) * (size_t)slots));
+  CK(cudaMemset(c.busy, 0, sizeof(int) * (size_t)slots));
+  CK(cudaMalloc(&c.work, sizeof(double) * (size_t)c.work_stride * (size_t)slots));
+  c.fn = fn;
   return JRLQP_OK;
 }
 
+// Calls of one family (cold / warm) take the large-n kernel: configured, and its workspace allocated, on first use
+static int use_large(jrlqp_solver * s, bool warm)
+{
+  LaunchCfg & c = s->large_cfg[warm];
+  if(!c.fn)
+  {
+    int rc = configure_large(s, warm, c);
+    if(rc != JRLQP_OK) return rc;
+  }
+  s->cfg[warm] = c;
+  return JRLQP_OK;
+}
+
+// Cold calls
 static int configure_kernel(jrlqp_solver * s)
 {
   if(s->n > 128 && s->path_mode == 1)
@@ -336,42 +351,13 @@ static int configure_kernel(jrlqp_solver * s)
     s->err = "the shared-memory kernel needs n <= 128";
     return JRLQP_ERR_ARG;
   }
-  s->large = s->path_mode == 2 || (s->path_mode == 0 && s->n > 128);
-  if(s->large)
-  {
-    int rc = configure_large(s, false);
-    if(rc != JRLQP_OK) return rc;
-    s->occ = s->locc[0];
-    s->smem_bytes = s->lsmem_bytes[0];
-    s->regs = s->lregs[0];
-    s->stage = false;
-    return JRLQP_OK;
-  }
+  if(s->path_mode == 2 || (s->path_mode == 0 && s->n > 128)) return use_large(s, false);
   // choose staging of C: automatic mode stages it when that costs no residency
-  auto try_cfg = [&](bool stage, int & occ, int & smem, KernelFn & fn, Layout & lay) -> int
-  {
-    lay = make_layout(s->n, s->mc, s->nb, s->warps, stage);
-    smem = lay.total_doubles * 8;
-    fn = pick_kernel(s->warps, stage);
-    occ = 0;
-    if(smem > s->max_smem_optin) return 0;
-    if(jrlqp::raise_smem_limit(fn, smem) != cudaSuccess)
-    {
-      cudaGetLastError();
-      return 0;
-    }
-    if(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, 32 * s->warps, smem) != cudaSuccess)
-    {
-      cudaGetLastError();
-      occ = 0;
-    }
-    return occ;
-  };
-  int occN = 0, occS = 0, smN = 0, smS = 0;
-  KernelFn fnN = nullptr, fnS = nullptr;
-  Layout layN{}, layS{};
-  try_cfg(false, occN, smN, fnN, layN);
-  if(s->mc > 0) try_cfg(true, occS, smS, fnS, layS);
+  const int threads = 32 * s->warps;
+  const DenseSmem layN = make_layout(s->n, s->mc, s->nb, s->warps, false), layS = make_layout(s->n, s->mc, s->nb, s->warps, true);
+  const int smN = layN.total_doubles * 8, smS = layS.total_doubles * 8;
+  const int occN = resident_ctas(s, pick_kernel(s->warps, false), threads, smN);
+  const int occS = s->mc > 0 ? resident_ctas(s, pick_kernel(s->warps, true), threads, smS) : 0;
   bool stage;
   if(s->stage_mode == 0)
     stage = false;
@@ -379,57 +365,71 @@ static int configure_kernel(jrlqp_solver * s)
     stage = occS > 0;
   else
     stage = occS > 0 && occS >= occN; // automatic: stage only when residency is not reduced
-  if(stage)
-  {
-    s->occ = occS;
-    s->smem_bytes = smS;
-    s->kernel = fnS;
-    s->lay = layS;
-  }
-  else
-  {
-    s->occ = occN;
-    s->smem_bytes = smN;
-    s->kernel = fnN;
-    s->lay = layN;
-  }
-  s->stage = stage;
-  if(s->warps == 3 && s->occ > 0)
+  KernelFn fn = pick_kernel(s->warps, stage);
+  int occ = stage ? occS : occN;
+  if(s->warps == 3 && occ > 0)
   {
     // register-capped instantiation of the three-warp kernel: taken when it makes more QPs resident (with C staged only
     // if that costs no residency, as above)
-    auto occ_of = [&](KernelFn fc, int smem) -> int
-    {
-      int o = 0;
-      if(smem <= 0 || smem > s->max_smem_optin) return 0;
-      if(jrlqp::raise_smem_limit(fc, smem) != cudaSuccess || cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, fc, 96, smem) != cudaSuccess)
-      {
-        cudaGetLastError();
-        return 0;
-      }
-      return o;
-    };
-    const int ocN = occ_of(gi_dense_cta_kernel<3, false, false, 4>, smN);
-    const int ocS = (s->stage_mode != 0 && occS > 0) ? occ_of(gi_dense_cta_kernel<3, true, false, 4>, smS) : 0;
+    const int ocN = resident_ctas(s, gi_dense_cta_kernel<3, false, false, 4>, threads, smN);
+    const int ocS = (s->stage_mode != 0 && occS > 0) ? resident_ctas(s, gi_dense_cta_kernel<3, true, false, 4>, threads, smS) : 0;
     const bool cstage = s->stage_mode == 1 ? ocS > 0 : (ocS > 0 && ocS >= ocN);
     const int occC = cstage ? ocS : ocN;
-    if(occC > s->occ)
+    if(occC > occ)
     {
-      s->occ = occC;
-      s->stage = cstage;
-      s->smem_bytes = cstage ? smS : smN;
-      s->lay = cstage ? layS : layN;
-      s->kernel = cstage ? (KernelFn)gi_dense_cta_kernel<3, true, false, 4> : (KernelFn)gi_dense_cta_kernel<3, false, false, 4>;
+      occ = occC;
+      stage = cstage;
+      fn = cstage ? (KernelFn)gi_dense_cta_kernel<3, true, false, 4> : (KernelFn)gi_dense_cta_kernel<3, false, false, 4>;
     }
   }
-  if(s->occ <= 0)
+  LaunchCfg & c = s->cfg[0];
+  c = LaunchCfg{};
+  c.fn = fn;
+  c.threads = threads;
+  c.smem = stage ? smS : smN;
+  c.occ = occ;
+  c.stage = stage;
+  c.lay = stage ? layS : layN;
+  if(occ <= 0)
   {
     s->err = "problem does not fit in shared memory (n too large for the dense warp kernel)";
     return JRLQP_ERR_ARG;
   }
   cudaFuncAttributes attr;
-  CK(cudaFuncGetAttributes(&attr, s->kernel));
-  s->regs = attr.numRegs;
+  CK(cudaFuncGetAttributes(&attr, fn));
+  c.regs = attr.numRegs;
+  return JRLQP_OK;
+}
+
+// Warm calls. In automatic mode a warm layout of the shared-memory kernel that does not fit (n >= ~116: n (n - 1) / 2 more
+// doubles than the cold one) sends the warm calls to the large-n kernel, which computes the same bits; cold calls keep the
+// shared-memory kernel.
+static int configure_warm(jrlqp_solver * s)
+{
+  if(s->cfg[1].fn) return JRLQP_OK;
+  if(s->cfg[0].large) return use_large(s, true);
+  const DenseSmem lay = make_layout(s->n, s->mc, s->nb, s->warps, false, true);
+  const int smem = lay.total_doubles * 8;
+  KernelFn fn = pick_warm_kernel(s->warps);
+  if(smem > s->max_smem_optin && s->path_mode == 0) return use_large(s, true);
+  if(!fn || smem > s->max_smem_optin)
+  {
+    s->err = "warm start: problem does not fit in shared memory (n too large; the Householder vectors need n (n - 1) / 2 more doubles)";
+    return JRLQP_ERR_ARG;
+  }
+  const int occ = resident_ctas(s, fn, 32 * s->warps, smem);
+  if(occ < 1)
+  {
+    s->err = "warm start kernel cannot be made resident";
+    return JRLQP_ERR_ARG;
+  }
+  LaunchCfg & c = s->cfg[1];
+  c = LaunchCfg{};
+  c.threads = 32 * s->warps;
+  c.smem = smem;
+  c.occ = occ;
+  c.lay = lay;
+  c.fn = fn;
   return JRLQP_OK;
 }
 
@@ -503,7 +503,7 @@ int jrlqp_destroy(jrlqp_solver * s)
 {
   if(!s) return JRLQP_OK;
   cudaSetDevice(s->device);
-  void * ptrs[] = {s->d_fcache, s->d_cts, s->d_pre, s->d_pre_ok, s->d_ct, s->d_ct_busy, s->d_seq_it, s->d_seq_status, s->d_seq, s->d_seq_tot, s->d_work[0], s->d_work[1], s->d_busy[0], s->d_busy[1], s->d_as, s->d_phase, s->d_counters, s->d_G, s->d_a, s->d_C, s->d_bl, s->d_bu, s->d_xl, s->d_xu, s->d_x, s->d_u, s->d_f, s->d_L,
+  void * ptrs[] = {s->d_fcache, s->d_cts, s->d_pre, s->d_pre_ok, s->d_ct, s->d_ct_busy, s->d_seq_it, s->d_seq_status, s->d_seq, s->d_seq_tot, s->large_cfg[0].work, s->large_cfg[1].work, s->large_cfg[0].busy, s->large_cfg[1].busy, s->d_as, s->d_phase, s->d_counters, s->d_G, s->d_a, s->d_C, s->d_bl, s->d_bu, s->d_xl, s->d_xu, s->d_x, s->d_u, s->d_f, s->d_L,
                    s->d_it, s->d_status, s->d_alist, s->d_nact, s->d_act};
   for(void * p : ptrs)
     if(p) cudaFree(p);
@@ -541,8 +541,7 @@ int jrlqp_set_kernel_path(jrlqp_solver * s, int32_t mode)
 {
   if(!s || mode < 0 || mode > 2) return JRLQP_ERR_ARG;
   s->path_mode = mode;
-  s->wkernel = nullptr;
-  s->warm_large = false;
+  s->cfg[1] = LaunchCfg{};
   cudaSetDevice(s->device);
   return configure_kernel(s);
 }
@@ -551,7 +550,7 @@ int64_t jrlqp_host_g_bytes(const jrlqp_solver * s, int32_t pinned)
 {
   if(!s) return 0;
   const long long n = s->n, h = n / 2;
-  if(pinned && !s->large && (g_zero_copy_G == 1 || (g_zero_copy_G < 0 && n <= 64))) return 8 * (n * (n + 1) / 2); // lower triangle, read in place
+  if(pinned && !s->cfg[0].large && (g_zero_copy_G == 1 || (g_zero_copy_G < 0 && n <= 64))) return 8 * (n * (n + 1) / 2); // lower triangle, read in place
   if(g_h2d_lower && n >= 32) return 8 * (n * h + (n - h) * (n - h)); // left columns + bottom-right block
   return 8 * n * n;
 }
@@ -566,14 +565,15 @@ int jrlqp_set_scan_transposed(jrlqp_solver * s, int32_t on)
 int jrlqp_get_kernel_info(const jrlqp_solver * s, jrlqp_kernel_info * info)
 {
   if(!s || !info) return JRLQP_ERR_ARG;
-  info->threads_per_qp = s->large ? kLargeThreads : 32 * s->warps;
-  info->rows_per_thread = s->large ? (s->n + kLargeThreads - 1) / kLargeThreads : 1;
-  info->smem_bytes_per_qp = s->smem_bytes;
-  info->qps_per_sm = s->occ;
-  info->grid = s->occ * s->num_sms;
+  const LaunchCfg & c = s->cfg[0];
+  info->threads_per_qp = c.threads;
+  info->rows_per_thread = c.large ? (s->n + kLargeThreads - 1) / kLargeThreads : 1;
+  info->smem_bytes_per_qp = c.smem;
+  info->qps_per_sm = c.occ;
+  info->grid = c.occ * s->num_sms;
   info->num_sms = s->num_sms;
-  info->stage_c = s->stage ? 1 : 0;
-  info->regs_per_thread = s->regs;
+  info->stage_c = c.stage ? 1 : 0;
+  info->regs_per_thread = c.regs;
   return JRLQP_OK;
 }
 
@@ -611,14 +611,12 @@ static int validate(const jrlqp_solver * s, const jrlqp_problem * pb, const jrlq
   return JRLQP_OK;
 }
 
-static int configure_warm(jrlqp_solver * s);
-
 // Large-n kernel, G shared by the batch (stride 0): Cholesky and J = L^-T are computed ONCE, by one CTA running the
 // solver's own factorisation code (same bits), and every solver CTA copies them instead of redoing 2/3 n^3 flops per
 // instance (the MultiIK fixtures of config C spend ~100 % of a solve there). Asynchronous on `st`.
 static bool uses_prefactor(const jrlqp_solver * s, const jrlqp_problem * pb, bool warm)
 {
-  return large_for(s, warm) && pb->G_stride == 0 && pb->batch >= 2;
+  return s->cfg[warm].large && pb->G_stride == 0 && pb->batch >= 2;
 }
 
 static int prefactor(jrlqp_solver * s, const jrlqp_problem * pb, cudaStream_t st)
@@ -650,7 +648,7 @@ static int prefactor(jrlqp_solver * s, const jrlqp_problem * pb, cudaStream_t st
 // Large-n kernel, C shared by the batch: one transposed copy per call for the coalesced constraint scan.
 static bool uses_shared_ct(const jrlqp_solver * s, const jrlqp_problem * pb, bool warm)
 {
-  return large_for(s, warm) && s->mc > 0 && pb->C_stride == 0 && pb->batch >= 2 && s->scan_transposed != 0;
+  return s->cfg[warm].large && s->mc > 0 && pb->C_stride == 0 && pb->batch >= 2 && s->scan_transposed != 0;
 }
 
 static int prepare_shared_ct(jrlqp_solver * s, const jrlqp_problem * pb, cudaStream_t st)
@@ -677,8 +675,8 @@ static bool scan_transposed_on(const jrlqp_solver * s)
 // (cold and warm, whatever the launch or stream) can be resident at the same time.
 static int ensure_ct(jrlqp_solver * s)
 {
-  if(s->large || s->mc == 0 || !scan_transposed_on(s)) return JRLQP_OK;
-  const int slots = 2 * std::max(s->occ, 1) * s->num_sms;
+  if(s->mc == 0 || !scan_transposed_on(s)) return JRLQP_OK;
+  const int slots = 2 * std::max(s->cfg[0].occ, 1) * s->num_sms;
   if(s->d_ct && slots <= s->ct_slots) return JRLQP_OK;
   if(s->d_ct) CK(cudaFree(s->d_ct));
   if(s->d_ct_busy) CK(cudaFree(s->d_ct_busy));
@@ -693,22 +691,15 @@ static int ensure_ct(jrlqp_solver * s)
   return JRLQP_OK;
 }
 
-static int launch(jrlqp_solver * s, const jrlqp_problem * pb, const jrlqp_result * res, cudaStream_t st, unsigned long long * counter, bool warm = false, bool force_warm_start = false,
-                  bool pre_ready = false)
+static int launch(jrlqp_solver * s, const jrlqp_problem * pb, const jrlqp_result * res, cudaStream_t st, unsigned long long * counter, const CallArgs & call)
 {
-  if(warm)
-  {
-    int rc = configure_warm(s); // (may set warm_large)
-    if(rc != JRLQP_OK) return rc;
-  }
-  const bool large = large_for(s, warm);
-  {
-    int rc = large ? configure_large(s, warm) : ensure_ct(s);
-    if(rc != JRLQP_OK) return rc;
-  }
-  const Layout & lay = warm ? s->wlay : s->lay;
+  const bool warm = call.warm;
+  int rc = warm ? configure_warm(s) : JRLQP_OK;
+  if(rc != JRLQP_OK) return rc;
+  const LaunchCfg & cfg = s->cfg[warm];
+  if(!cfg.large && (rc = ensure_ct(s)) != JRLQP_OK) return rc;
   GiParams p{};
-  if(!large && s->mc > 0 && scan_transposed_on(s) && s->d_ct)
+  if(!cfg.large && s->mc > 0 && scan_transposed_on(s) && s->d_ct)
   {
     p.ct = s->d_ct;
     p.ct_stride = s->ct_stride;
@@ -740,7 +731,7 @@ static int launch(jrlqp_solver * s, const jrlqp_problem * pb, const jrlqp_result
   p.sxu = pb->xu_stride;
   p.as_in = warm ? reinterpret_cast<const signed char *>(pb->as_in) : nullptr;
   p.s_as = pb->as_stride;
-  p.warm_start = warm ? (force_warm_start ? 1 : s->opt.warm_start) : 0;
+  p.warm_start = warm ? (call.force_warm_start ? 1 : s->opt.warm_start) : 0;
   p.x = res->x;
   p.u = res->u;
   p.f = res->f;
@@ -752,112 +743,33 @@ static int launch(jrlqp_solver * s, const jrlqp_problem * pb, const jrlqp_result
   p.L = res->L;
   p.counter = counter;
   p.phase_cycles = s->d_phase;
-  p.ldj = lay.ldj;
-  p.ldcs = lay.ldcs;
-  p.npad = lay.npad;
-  p.off_R = lay.off_R;
-  p.off_x = lay.off_x;
-  p.off_z = lay.off_z;
-  p.off_d = lay.off_d;
-  p.off_r = lay.off_r;
-  p.off_u = lay.off_u;
-  p.off_cv = lay.off_cv;
-  p.off_gc = lay.off_gc;
-  p.off_gs = lay.off_gs;
-  p.off_gcs = lay.off_gcs;
-  p.off_ldiag = lay.off_ldiag;
-  p.off_rinv = lay.off_rinv;
-  p.off_scr = lay.off_scr;
-  p.off_C = lay.off_C;
-  p.off_alist = lay.off_alist;
-  p.off_gk = lay.off_gk;
-  p.off_iscr = lay.off_iscr;
-  p.off_stat = lay.off_stat;
-  p.off_eq = lay.off_eq;
-  p.off_il = lay.off_il;
-  p.off_V = lay.off_V;
-  p.off_bact = lay.off_bact;
-  p.off_hco = lay.off_hco;
-  p.off_alpha = lay.off_alpha;
+  p.lay = cfg.lay;
   p.fcache = s->d_fcache;
   p.fcache_stride = (long long)s->n * s->n + 2ll * s->n;
-  p.fcache_mode = (warm && !large && s->d_fcache != nullptr) ? s->fcache_mode : 0;
-  const int occ = large ? s->locc[warm ? 1 : 0] : (warm ? s->wocc : s->occ);
-  long long grid = std::min<long long>((long long)occ * s->num_sms, std::max<long long>(pb->batch, 1));
+  p.fcache_mode = call.fcache_mode;
+  p.work = cfg.work;
+  p.work_stride = cfg.work_stride;
+  p.work_busy = cfg.busy;
+  p.work_slots = cfg.work_slots;
+  p.ring_cols = cfg.ring_cols;
+  p.slab_rows = cfg.slab_rows;
+  long long grid = std::min<long long>((long long)cfg.occ * s->num_sms, std::max<long long>(pb->batch, 1));
   CK(cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st));
   if(uses_prefactor(s, pb, warm))
   {
-    if(!pre_ready)
-    {
-      int rc = prefactor(s, pb, st);
-      if(rc != JRLQP_OK) return rc;
-    }
+    if(!call.pre_ready && (rc = prefactor(s, pb, st)) != JRLQP_OK) return rc;
     p.pre = s->d_pre;
     p.pre_ok = s->d_pre_ok;
   }
   if(uses_shared_ct(s, pb, warm))
   {
-    if(!pre_ready)
-    {
-      int rc = prepare_shared_ct(s, pb, st);
-      if(rc != JRLQP_OK) return rc;
-    }
+    if(!call.pre_ready && (rc = prepare_shared_ct(s, pb, st)) != JRLQP_OK) return rc;
     p.ct = s->d_cts;
     p.ldct = s->ldcts;
   }
-  if(large)
-  {
-    p.work = s->d_work[warm ? 1 : 0];
-    p.work_stride = s->work_stride[warm ? 1 : 0];
-    p.work_busy = s->d_busy[warm ? 1 : 0];
-    p.work_slots = s->work_slots[warm ? 1 : 0];
-    p.ring_cols = s->lring[warm ? 1 : 0];
-    p.slab_rows = warm ? s->lslab : 0;
-    if(warm)
-      gi_large_kernel<kLargeThreads, true><<<(unsigned)grid, kLargeThreads, s->lsmem_bytes[1], st>>>(p);
-    else
-      gi_large_kernel<kLargeThreads, false><<<(unsigned)grid, kLargeThreads, s->lsmem_bytes[0], st>>>(p);
-  }
-  else if(warm)
-    s->wkernel<<<(unsigned)grid, 32 * s->warps, s->wsmem_bytes, st>>>(p);
-  else
-    s->kernel<<<(unsigned)grid, 32 * s->warps, s->smem_bytes, st>>>(p);
+  cfg.fn<<<(unsigned)grid, cfg.threads, cfg.smem, st>>>(p);
   g_launches.fetch_add(1);
   CK(cudaGetLastError());
-  return JRLQP_OK;
-}
-
-// Shared-memory warm kernel, for handles whose cold calls take the shared-memory kernel. In automatic mode a warm layout
-// that does not fit (n >= ~116: n (n - 1) / 2 more doubles than the cold one) sends the warm calls to the large-n kernel,
-// which computes the same bits; cold calls keep the shared-memory kernel.
-static int configure_warm(jrlqp_solver * s)
-{
-  if(s->large || s->wkernel || s->warm_large) return JRLQP_OK;
-  Layout lay = make_layout(s->n, s->mc, s->nb, s->warps, false, true);
-  const int smem = lay.total_doubles * 8;
-  KernelFn fn = pick_warm_kernel(s->warps);
-  if(smem > s->max_smem_optin && s->path_mode == 0)
-  {
-    s->warm_large = true;
-    return JRLQP_OK;
-  }
-  if(!fn || smem > s->max_smem_optin)
-  {
-    s->err = "warm start: problem does not fit in shared memory (n too large; the Householder vectors need n (n - 1) / 2 more doubles)";
-    return JRLQP_ERR_ARG;
-  }
-  CK(jrlqp::raise_smem_limit(fn, smem));
-  int occ = 0;
-  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, 32 * s->warps, smem));
-  if(occ < 1)
-  {
-    s->err = "warm start kernel cannot be made resident";
-    return JRLQP_ERR_ARG;
-  }
-  s->wlay = lay;
-  s->wsmem_bytes = smem;
-  s->wocc = occ;
-  s->wkernel = fn;
   return JRLQP_OK;
 }
 
@@ -885,7 +797,7 @@ int jrlqp_solve_batch_warm_device(jrlqp_solver * s, const jrlqp_problem * pb, co
   CK(cudaSetDevice(s->device));
   unsigned long long * counter = s->d_counters + (s->next_counter++ % kMaxChunks);
   if((rc = serialise_begin(s, (cudaStream_t)stream)) != JRLQP_OK) return rc;
-  rc = launch(s, pb, res, (cudaStream_t)stream, counter, true);
+  rc = launch(s, pb, res, (cudaStream_t)stream, counter, CallArgs{true});
   if(rc != JRLQP_OK) return rc;
   return serialise_end(s, (cudaStream_t)stream);
 }
@@ -898,7 +810,7 @@ int jrlqp_solve_batch_device(jrlqp_solver * s, const jrlqp_problem * pb, const j
   CK(cudaSetDevice(s->device));
   unsigned long long * counter = s->d_counters + (s->next_counter++ % kMaxChunks);
   if((rc = serialise_begin(s, (cudaStream_t)stream)) != JRLQP_OK) return rc;
-  rc = launch(s, pb, res, (cudaStream_t)stream, counter);
+  rc = launch(s, pb, res, (cudaStream_t)stream, counter, CallArgs{});
   if(rc != JRLQP_OK) return rc;
   return serialise_end(s, (cudaStream_t)stream);
 }
@@ -990,6 +902,68 @@ static cudaError_t h2d_G(double * dst, const double * src, long long stride, lon
   return cudaMemcpy3DAsync(&p3, st);
 }
 
+enum : int
+{
+  kStageShared = 1, // arrays shared by the batch (stride 0): one slot each
+  kStageInstances = 2 // the other arrays, and as_in
+};
+
+// Fills `dp` with the device copy, in the handle's staging, of instances [b0, b0 + cnt) of the caller's host problem `pb`,
+// and enqueues on `st` the copies of the arrays `which` selects. Arrays left null in `pb` are not staged. G crosses whole,
+// or in the two-block layout of h2d_G with `lower_G`, or not at all when `mapped_G` (the device alias of the caller's
+// pinned G, read in place by the kernels) is given.
+static int stage_host_problem(jrlqp_solver * s, const jrlqp_problem * pb, long long b0, long long cnt, int which, bool lower_G,
+                              const double * mapped_G, cudaStream_t st, jrlqp_problem * dp)
+{
+  const long long n = s->n, mc = s->mc, m = s->m;
+  auto up = [&](double * dbase, const double * h, long long hstride, int rows, int cols, int ld, const double *& dptr, int64_t & dstride,
+                bool lower = false) -> cudaError_t
+  {
+    if(!h) return cudaSuccess;
+    const long long blk = (long long)rows * cols;
+    double * d = hstride == 0 ? dbase : dbase + b0 * blk;
+    dptr = d;
+    dstride = hstride == 0 ? 0 : blk;
+    if(!(which & (hstride == 0 ? kStageShared : kStageInstances))) return cudaSuccess;
+    return lower ? h2d_G(d, h + b0 * hstride, hstride, cnt, rows, ld, st) : h2d(d, h + b0 * hstride, hstride, cnt, rows, cols, ld, st);
+  };
+  dp->batch = cnt;
+  if(mapped_G)
+  {
+    dp->G = mapped_G + b0 * pb->G_stride;
+    dp->G_stride = pb->G_stride;
+  }
+  else
+    CK(up(s->d_G, pb->G, pb->G_stride, (int)n, (int)n, pb->ldg, dp->G, dp->G_stride, lower_G));
+  dp->ldg = mapped_G ? pb->ldg : (int)n;
+  CK(up(s->d_a, pb->a, pb->a_stride, (int)n, 1, (int)n, dp->a, dp->a_stride));
+  if(mc)
+  {
+    CK(up(s->d_C, pb->C, pb->C_stride, (int)n, (int)mc, pb->ldc, dp->C, dp->C_stride));
+    CK(up(s->d_bl, pb->bl, pb->bl_stride, (int)mc, 1, (int)mc, dp->bl, dp->bl_stride));
+    CK(up(s->d_bu, pb->bu, pb->bu_stride, (int)mc, 1, (int)mc, dp->bu, dp->bu_stride));
+  }
+  dp->ldc = (int)n;
+  if(s->nb)
+  {
+    CK(up(s->d_xl, pb->xl, pb->xl_stride, (int)n, 1, (int)n, dp->xl, dp->xl_stride));
+    CK(up(s->d_xu, pb->xu, pb->xu_stride, (int)n, 1, (int)n, dp->xu, dp->xu_stride));
+  }
+  if(pb->as_in && (which & kStageInstances))
+  {
+    if(!s->d_as) CK(cudaMalloc(&s->d_as, std::max<long long>(std::max<long long>(s->capacity, 1) * m, 1)));
+    const long long cnt_as = pb->as_stride == 0 ? 1 : cnt;
+    signed char * das = s->d_as + b0 * m;
+    if(pb->as_stride == m || cnt_as == 1)
+      CK(cudaMemcpyAsync(das, pb->as_in + b0 * pb->as_stride, (size_t)(cnt_as * m), cudaMemcpyHostToDevice, st));
+    else
+      CK(cudaMemcpy2DAsync(das, (size_t)m, pb->as_in + b0 * pb->as_stride, (size_t)pb->as_stride, (size_t)m, (size_t)cnt_as, cudaMemcpyHostToDevice, st));
+    dp->as_in = reinterpret_cast<const int8_t *>(das);
+    dp->as_stride = pb->as_stride == 0 ? 0 : m;
+  }
+  return JRLQP_OK;
+}
+
 static int solve_batch_host_impl(jrlqp_solver * s, const jrlqp_problem * pb, const jrlqp_result * res, bool warm)
 {
   int rc = validate(s, pb, res);
@@ -1000,7 +974,6 @@ static int solve_batch_host_impl(jrlqp_solver * s, const jrlqp_problem * pb, con
   rc = ensure_staging(s, pb, res->L != nullptr);
   if(rc != JRLQP_OK) return rc;
   if(warm && (rc = configure_warm(s)) != JRLQP_OK) return rc;
-  const bool large = large_for(s, warm);
 
   const long long B = pb->batch;
   const long long n = s->n, mc = s->mc, m = s->m;
@@ -1008,7 +981,7 @@ static int solve_batch_host_impl(jrlqp_solver * s, const jrlqp_problem * pb, con
   // GPU), the kernels read G straight from the caller's PINNED buffer: only the lower triangle crosses PCIe, as
   // SM-initiated reads concurrent with the DMA of the other arrays (measured, profiles/r01u_*: +5 % at n = 50, +9 % at
   // n = 20 over the two-block upload, -5 % at n = 128, which is kernel-bound: automatic mode = n <= 64).
-  const bool zero_copy_G = !large && !res->L && pb->G_stride != 0 && (g_zero_copy_G == 1 || (g_zero_copy_G < 0 && s->n <= 64));
+  const bool zero_copy_G = !s->cfg[warm].large && !res->L && pb->G_stride != 0 && (g_zero_copy_G == 1 || (g_zero_copy_G < 0 && s->n <= 64));
   const double * g_dev_ptr_G = nullptr;
   if(zero_copy_G)
   {
@@ -1021,7 +994,7 @@ static int solve_batch_host_impl(jrlqp_solver * s, const jrlqp_problem * pb, con
   // Pipeline: split the batch into chunks; chunk c runs H2D -> kernel -> D2H on stream c % kStreams,
   // so the copy engines and the SMs overlap across chunks.
   const long long per_qp_bytes = 8 * (n * n + n + mc * n + 2 * mc + 2 * s->nb);
-  long long chunk = std::max<long long>((long long)s->occ * s->num_sms * 4, (48ll << 20) / std::max<long long>(per_qp_bytes, 1));
+  long long chunk = std::max<long long>((long long)s->cfg[0].occ * s->num_sms * 4, (48ll << 20) / std::max<long long>(per_qp_bytes, 1));
   long long nchunks = std::min<long long>(kMaxChunks, std::max<long long>(1, (B + chunk - 1) / chunk));
   if(const char * e = getenv("JRLQP_HOST_CHUNK")) // tuning: QPs per chunk of the host pipeline (scripts/e2e_chunk_sweep.py)
   {
@@ -1030,56 +1003,21 @@ static int solve_batch_host_impl(jrlqp_solver * s, const jrlqp_problem * pb, con
   }
   chunk = (B + nchunks - 1) / nchunks;
 
-  // arrays shared by the batch (stride 0): uploaded once, on stream 0; the other streams wait for them
+  jrlqp_problem hp = *pb;
+  if(!warm) hp.as_in = nullptr; // (read by warm calls only)
+  const bool lower_G = !res->L; // (the factor copy-out reads nothing of G's upper part either, but keep it simple)
+  // arrays shared by the batch (stride 0): uploaded once, on stream 0, with the factor of a shared G and the transposed copy
+  // of a shared C that all the chunks re-use; the other streams wait for them
+  if(pb->G_stride == 0 || pb->a_stride == 0 || (mc && (pb->C_stride == 0 || pb->bl_stride == 0 || pb->bu_stride == 0))
+     || (s->nb && (pb->xl_stride == 0 || pb->xu_stride == 0)))
   {
-    bool any = false;
-    auto up1 = [&](double * d, const double * h, long long hstride, int rows, int cols, int ld) -> cudaError_t
-    {
-      if(hstride != 0 || !h) return cudaSuccess;
-      any = true;
-      return h2d(d, h, 0, 1, rows, cols, ld, s->streams[0]);
-    };
-    CK(up1(s->d_G, pb->G, pb->G_stride, (int)n, (int)n, pb->ldg));
-    CK(up1(s->d_a, pb->a, pb->a_stride, (int)n, 1, (int)n));
-    if(mc)
-    {
-      CK(up1(s->d_C, pb->C, pb->C_stride, (int)n, (int)mc, pb->ldc));
-      CK(up1(s->d_bl, pb->bl, pb->bl_stride, (int)mc, 1, (int)mc));
-      CK(up1(s->d_bu, pb->bu, pb->bu_stride, (int)mc, 1, (int)mc));
-    }
-    if(s->nb)
-    {
-      CK(up1(s->d_xl, pb->xl, pb->xl_stride, (int)n, 1, (int)n));
-      CK(up1(s->d_xu, pb->xu, pb->xu_stride, (int)n, 1, (int)n));
-    }
-    if(large && pb->G_stride == 0 && B >= 2)
-    {
-      // factor of the shared G, once for the whole call (the chunks below re-use it)
-      jrlqp_problem pg{};
-      pg.batch = B;
-      pg.G = s->d_G;
-      pg.G_stride = 0;
-      pg.ldg = (int)n;
-      pg.ldc = (int)n;
-      int rcp = prefactor(s, &pg, s->streams[0]);
-      if(rcp != JRLQP_OK) return rcp;
-    }
-    if(large && mc > 0 && pb->C_stride == 0 && B >= 2 && s->scan_transposed != 0)
-    {
-      jrlqp_problem pc{};
-      pc.batch = B;
-      pc.C = s->d_C;
-      pc.C_stride = 0;
-      pc.ldc = (int)n;
-      int rcc = prepare_shared_ct(s, &pc, s->streams[0]);
-      if(rcc != JRLQP_OK) return rcc;
-    }
-    if(any)
-    {
-      if(!s->ev_shared) CK(cudaEventCreateWithFlags(&s->ev_shared, cudaEventDisableTiming));
-      CK(cudaEventRecord(s->ev_shared, s->streams[0]));
-      for(int i = 1; i < kStreams; ++i) CK(cudaStreamWaitEvent(s->streams[i], s->ev_shared, 0));
-    }
+    jrlqp_problem dsh{};
+    if((rc = stage_host_problem(s, &hp, 0, B, kStageShared, lower_G, g_dev_ptr_G, s->streams[0], &dsh)) != JRLQP_OK) return rc;
+    if(uses_prefactor(s, &dsh, warm) && (rc = prefactor(s, &dsh, s->streams[0])) != JRLQP_OK) return rc;
+    if(uses_shared_ct(s, &dsh, warm) && (rc = prepare_shared_ct(s, &dsh, s->streams[0])) != JRLQP_OK) return rc;
+    if(!s->ev_shared) CK(cudaEventCreateWithFlags(&s->ev_shared, cudaEventDisableTiming));
+    CK(cudaEventRecord(s->ev_shared, s->streams[0]));
+    for(int i = 1; i < kStreams; ++i) CK(cudaStreamWaitEvent(s->streams[i], s->ev_shared, 0));
   }
 
   for(long long c = 0; c < nchunks; ++c)
@@ -1089,52 +1027,7 @@ static int solve_batch_host_impl(jrlqp_solver * s, const jrlqp_problem * pb, con
     if(cnt <= 0) break;
     cudaStream_t st = s->streams[c % kStreams];
     jrlqp_problem dp{};
-    dp.batch = cnt;
-    auto up = [&](double * dbase, const double * h, long long hstride, int rows, int cols, int ld, const double *& dptr, int64_t & dstride) -> cudaError_t
-    {
-      const long long blk = (long long)rows * cols;
-      if(hstride == 0)
-      {
-        dptr = dbase; // uploaded above
-        dstride = 0;
-        return cudaSuccess;
-      }
-      double * d = dbase + b0 * blk;
-      dptr = d;
-      dstride = blk;
-      return h2d(d, h + b0 * hstride, hstride, cnt, rows, cols, ld, st);
-    };
-    if(g_dev_ptr_G != nullptr)
-    {
-      // G is read by the kernels straight from the caller's pinned host buffer (lower triangle only: about half the
-      // bytes of G cross PCIe, as SM-initiated reads that overlap the DMA of the other arrays)
-      dp.G = g_dev_ptr_G + b0 * pb->G_stride;
-      dp.G_stride = pb->G_stride;
-    }
-    else if(pb->G_stride != 0 && !res->L)
-    {
-      // lower-triangle-only upload (the factor copy-out reads nothing of G's upper part either, but keep it simple)
-      double * d = s->d_G + b0 * n * n;
-      dp.G = d;
-      dp.G_stride = n * n;
-      CK(h2d_G(d, pb->G + b0 * pb->G_stride, pb->G_stride, cnt, (int)n, pb->ldg, st));
-    }
-    else
-      CK(up(s->d_G, pb->G, pb->G_stride, (int)n, (int)n, pb->ldg, dp.G, dp.G_stride));
-    dp.ldg = g_dev_ptr_G != nullptr ? pb->ldg : (int)n;
-    CK(up(s->d_a, pb->a, pb->a_stride, (int)n, 1, (int)n, dp.a, dp.a_stride));
-    if(mc)
-    {
-      CK(up(s->d_C, pb->C, pb->C_stride, (int)n, (int)mc, pb->ldc, dp.C, dp.C_stride));
-      CK(up(s->d_bl, pb->bl, pb->bl_stride, (int)mc, 1, (int)mc, dp.bl, dp.bl_stride));
-      CK(up(s->d_bu, pb->bu, pb->bu_stride, (int)mc, 1, (int)mc, dp.bu, dp.bu_stride));
-    }
-    dp.ldc = (int)n;
-    if(s->nb)
-    {
-      CK(up(s->d_xl, pb->xl, pb->xl_stride, (int)n, 1, (int)n, dp.xl, dp.xl_stride));
-      CK(up(s->d_xu, pb->xu, pb->xu_stride, (int)n, 1, (int)n, dp.xu, dp.xu_stride));
-    }
+    if((rc = stage_host_problem(s, &hp, b0, cnt, kStageInstances, lower_G, g_dev_ptr_G, st, &dp)) != JRLQP_OK) return rc;
     jrlqp_result dr{};
     dr.x = s->d_x + b0 * n;
     dr.u = res->u ? s->d_u + b0 * m : nullptr;
@@ -1145,19 +1038,7 @@ static int solve_batch_host_impl(jrlqp_solver * s, const jrlqp_problem * pb, con
     dr.active_list = res->active_list ? s->d_alist + b0 * n : nullptr;
     dr.n_active = res->n_active ? s->d_nact + b0 : nullptr;
     dr.L = res->L ? s->d_L + b0 * n * n : nullptr;
-    if(warm && pb->as_in)
-    {
-      if(!s->d_as) CK(cudaMalloc(&s->d_as, std::max<long long>(std::max<long long>(s->capacity, 1) * m, 1)));
-      const long long cnt_as = pb->as_stride == 0 ? 1 : cnt;
-      signed char * das = s->d_as + b0 * m;
-      if(pb->as_stride == m || cnt_as == 1)
-        CK(cudaMemcpyAsync(das, pb->as_in + b0 * pb->as_stride, (size_t)(cnt_as * m), cudaMemcpyHostToDevice, st));
-      else
-        CK(cudaMemcpy2DAsync(das, (size_t)m, pb->as_in + b0 * pb->as_stride, (size_t)pb->as_stride, (size_t)m, (size_t)cnt_as, cudaMemcpyHostToDevice, st));
-      dp.as_in = reinterpret_cast<const int8_t *>(das);
-      dp.as_stride = pb->as_stride == 0 ? 0 : m;
-    }
-    rc = launch(s, &dp, &dr, st, s->d_counters + (c % kMaxChunks), warm, false, /*pre_ready=*/large); // shared factor / transposed C prepared above, once for all the chunks
+    rc = launch(s, &dp, &dr, st, s->d_counters + (c % kMaxChunks), CallArgs{warm, false, /*pre_ready=*/true}); // shared factor / transposed C prepared above
     if(rc != JRLQP_OK) return rc;
     CK(cudaMemcpyAsync(res->x + b0 * n, dr.x, sizeof(double) * cnt * n, cudaMemcpyDeviceToHost, st));
     if(res->u && m) CK(cudaMemcpyAsync(res->u + b0 * m, dr.u, sizeof(double) * cnt * m, cudaMemcpyDeviceToHost, st));
@@ -1236,7 +1117,7 @@ static int sequence_device_impl(jrlqp_solver * s, const jrlqp_problem * pb, cons
     if(rc != JRLQP_OK) return rc;
   }
   // G is the same at every step: the warm kernels keep the factor of step 0 in HBM and re-read it afterwards (same bits)
-  const bool use_fcache = seq->warm != 0 && !large_for(s, true) && seq->steps > 1 && !res->L && g_seq_fcache != 0;
+  const bool use_fcache = seq->warm != 0 && !s->cfg[1].large && seq->steps > 1 && !res->L && g_seq_fcache != 0;
   if(use_fcache)
   {
     const long long need = B * ((long long)s->n * s->n + 2ll * s->n);
@@ -1254,7 +1135,7 @@ static int sequence_device_impl(jrlqp_solver * s, const jrlqp_problem * pb, cons
   unsigned long long * counter = s->d_counters + (s->next_counter++ % kMaxChunks);
   for(int t = 0; t < seq->steps; ++t)
   {
-    s->fcache_mode = (use_fcache && s->d_fcache != nullptr && B * ((long long)s->n * s->n + 2ll * s->n) <= s->fcache_cap) ? (t == 0 ? 1 : 2) : 0;
+    const int fcache_mode = (use_fcache && s->d_fcache != nullptr && B * ((long long)s->n * s->n + 2ll * s->n) <= s->fcache_cap) ? (t == 0 ? 1 : 2) : 0;
     jrlqp_problem p = *pb;
     p.a = pb->a + (long long)t * seq->a_step_stride;
     jrlqp_result r = *res;
@@ -1275,8 +1156,7 @@ static int sequence_device_impl(jrlqp_solver * s, const jrlqp_problem * pb, cons
       p.as_in = res->active_set;
       p.as_stride = s->m;
     }
-    int rc = launch(s, &p, &r, st, counter, seq->warm != 0, seq->warm != 0, /*pre_ready=*/t > 0);
-    s->fcache_mode = 0;
+    int rc = launch(s, &p, &r, st, counter, CallArgs{seq->warm != 0, seq->warm != 0, /*pre_ready=*/t > 0, fcache_mode});
     if(rc != JRLQP_OK) return rc;
     if(totals)
     {
@@ -1311,7 +1191,7 @@ int jrlqp_solve_sequence_host(jrlqp_solver * s, const jrlqp_problem * pb, const 
   CK(cudaSetDevice(s->device));
   rc = ensure_staging(s, pb, false);
   if(rc != JRLQP_OK) return rc;
-  const long long B = pb->batch, n = s->n, mc = s->mc, m = s->m, T = seq->steps;
+  const long long B = pb->batch, n = s->n, m = s->m, T = seq->steps;
   cudaStream_t st = s->streams[0];
   // arena: [T][B][n] linear terms, then the per-step outputs that were asked for
   const long long na = T * B * n;
@@ -1337,28 +1217,11 @@ int jrlqp_solve_sequence_host(jrlqp_solver * s, const jrlqp_problem * pb, const 
   int * d_is = reinterpret_cast<int *>(d_fs + nf);
   int * d_ss = reinterpret_cast<int *>(d_fs + nf + ni);
 
+  jrlqp_problem hp = *pb;
+  hp.a = nullptr; // (the linear terms of every step go to the arena, below)
+  if(!seq->warm) hp.as_in = nullptr;
   jrlqp_problem dp{};
-  dp.batch = B;
-  auto up = [&](double * d, const double * h, long long hstride, int rows, int cols, int ld, const double *& dptr, int64_t & dstride) -> cudaError_t
-  {
-    dptr = d;
-    dstride = hstride == 0 ? 0 : (long long)rows * cols;
-    return h2d(d, h, hstride, B, rows, cols, ld, st);
-  };
-  CK(up(s->d_G, pb->G, pb->G_stride, (int)n, (int)n, pb->ldg, dp.G, dp.G_stride));
-  dp.ldg = (int)n;
-  dp.ldc = (int)n;
-  if(mc)
-  {
-    CK(up(s->d_C, pb->C, pb->C_stride, (int)n, (int)mc, pb->ldc, dp.C, dp.C_stride));
-    CK(up(s->d_bl, pb->bl, pb->bl_stride, (int)mc, 1, (int)mc, dp.bl, dp.bl_stride));
-    CK(up(s->d_bu, pb->bu, pb->bu_stride, (int)mc, 1, (int)mc, dp.bu, dp.bu_stride));
-  }
-  if(s->nb)
-  {
-    CK(up(s->d_xl, pb->xl, pb->xl_stride, (int)n, 1, (int)n, dp.xl, dp.xl_stride));
-    CK(up(s->d_xu, pb->xu, pb->xu_stride, (int)n, 1, (int)n, dp.xu, dp.xu_stride));
-  }
+  if((rc = stage_host_problem(s, &hp, 0, B, kStageShared | kStageInstances, false, nullptr, st, &dp)) != JRLQP_OK) return rc;
   // linear terms: step t, instance b at a + t * a_step_stride + b * a_stride  ->  dense [T][B][n]
   for(long long t = 0; t < T; ++t)
   {
@@ -1370,17 +1233,6 @@ int jrlqp_solve_sequence_host(jrlqp_solver * s, const jrlqp_problem * pb, const 
   }
   dp.a = d_aseq;
   dp.a_stride = n;
-  if(seq->warm && pb->as_in)
-  {
-    if(!s->d_as) CK(cudaMalloc(&s->d_as, std::max<long long>(std::max<long long>(s->capacity, 1) * m, 1)));
-    const long long cnt_as = pb->as_stride == 0 ? 1 : B;
-    if(pb->as_stride == m || cnt_as == 1)
-      CK(cudaMemcpyAsync(s->d_as, pb->as_in, (size_t)(cnt_as * m), cudaMemcpyHostToDevice, st));
-    else
-      CK(cudaMemcpy2DAsync(s->d_as, (size_t)m, pb->as_in, (size_t)pb->as_stride, (size_t)m, (size_t)cnt_as, cudaMemcpyHostToDevice, st));
-    dp.as_in = reinterpret_cast<const int8_t *>(s->d_as);
-    dp.as_stride = pb->as_stride == 0 ? 0 : m;
-  }
   jrlqp_sequence ds = *seq;
   ds.a_step_stride = B * n;
   ds.x_step_stride = nx ? B * n : 0;

@@ -28,6 +28,22 @@ enum : int
   TS_UNKNOWN = 7
 };
 
+// Shared-memory layout of the dense kernels (gi_dense_cta.cuh), computed on the host (capi.cu: make_layout); in doubles
+// unless noted. The offset of each field within the parameter block decides how the compiler pairs the kernels' 64- and
+// 128-bit loads of them: `pad` and the place of total_doubles keep those offsets, and so the kernels' machine code.
+struct DenseSmem
+{
+  int ldj; // leading dimension of the row-major J/L buffer (odd => conflict-free row-strided access)
+  int ldcs; // leading dimension of the staged C (odd), if staged
+  int npad; // threads per CTA (>= n)
+  int off_R, off_x, off_z, off_d, off_r, off_u, off_cv;
+  int pad[2];
+  int off_gcs, off_ldiag, off_rinv, off_scr, off_C, off_alist;
+  int total_doubles; // (host only)
+  int off_iscr, off_stat, off_eq, off_il; // int / int8 / uint16 arrays
+  int off_V, off_bact, off_hco, off_alpha; // warm-start kernels only
+};
+
 struct GiParams
 {
   // sizes
@@ -95,13 +111,7 @@ struct GiParams
   // persistent work queue
   unsigned long long * counter;
   unsigned long long * phase_cycles; // [4 warps][16 phases], only with -DJRLQP_PHASE_TIMING (else null)
-  // shared-memory layout (computed on the host, in doubles unless noted)
-  int ldj; // leading dimension of the row-major J/L buffer (odd => conflict-free row-strided access)
-  int ldcs; // leading dimension of the staged C (odd), if staged
-  int npad; // threads per CTA (>= n)
-  int off_R, off_x, off_z, off_d, off_r, off_u, off_cv, off_gc, off_gs, off_gcs, off_ldiag, off_rinv, off_scr, off_C; // offsets in doubles
-  int off_alist, off_gk, off_iscr, off_stat, off_eq, off_il;
-  int off_V, off_bact, off_hco, off_alpha; // warm-start kernels only (offsets in doubles) // offsets in doubles of the int / int8 arrays
+  DenseSmem lay; // dense kernels only
 };
 
 } // namespace jrlqp
