@@ -427,6 +427,9 @@ int jrlqp_structured_get_info(const jrlqp_structured * s, jrlqp_structured_info 
  * that no constraint is active after the initial scan (BlockGISolver.cpp:474); an instance whose data contain
  * bl == bu or xl == xu is reported as JRLQP_INCONSISTENT_INPUT. Instances that exhaust the storage of the
  * orthonormal sequence (2 n max_iter doubles per resident CTA) report JRLQP_UNKNOWN.
+ * Sizes: n <= 1024 variables, diagonal blocks of 1 ... 96 rows; jrlqp_blockgi_create returns JRLQP_ERR_ARG for a
+ * larger n, and for a problem whose per-CTA state (which grows with n, the largest block and max_iter) does not fit
+ * in the shared memory of one CTA.
  * --------------------------------------------------------------------------------------------- */
 
 /* structured::StructuredC(std::vector<MatrixConstRef>) (src/structured/StructuredC.cpp:9-25): block-diagonal

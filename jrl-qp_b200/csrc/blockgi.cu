@@ -131,6 +131,13 @@ int jrlqp_blockgi_create(jrlqp_blockgi ** out, const jrlqp_structure * G, const 
     return rc;
   }
   s->n = s->g->n;
+  if(s->n > 1024)
+  {
+    // the passes over Q hold entries tid + 128 j, j < 8, of a reflector and of the vector: entries past 1023 would never be
+    // updated (blockgi_kernel<8>, blockgi.cuh)
+    s->err = "n = " + std::to_string(s->n) + " exceeds 1024, the largest size the structured solver supports";
+    return JRLQP_ERR_ARG;
+  }
   s->cb = C->nblocks;
   int nv = 0, nc = 0;
   for(int i = 0; i < s->cb; ++i)

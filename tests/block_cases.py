@@ -5,6 +5,7 @@ block-diagonal C with double-sided inequalities built per block around a planted
 MultiIK fixtures split into blocks the way the tests do (:190-215, :286-303)."""
 import os
 import sys
+import types
 
 import numpy as np
 
@@ -74,6 +75,13 @@ def random_block_problem(type, sizes, mi, batch, seed, bounds=False, active_frac
     pb = BlockProblem(stG, stC, Gdata, a, Cdata, bl, bu, xl, xu, Gdense=H, Cdense=Cd)
     pb.x_planted = x0
     return pb
+
+
+def dense_view(pb):
+    """The dense copies of a batch with the attributes of a problems.ProblemBatch (G, a, C, bounds, mc), as
+    tests/test_warm_kkt_reference.py reads them; C is None without constraints."""
+    return types.SimpleNamespace(G=pb.Gdense, a=pb.a, C=pb.Cdense if pb.mc else None, bl=pb.bl, bu=pb.bu, xl=pb.xl, xu=pb.xu,
+                                 mc=pb.mc)
 
 
 def dense_solution(pb, nthreads=4):

@@ -215,6 +215,8 @@ def block_problem(which, s=1.0):
         pb = bc.random_block_problem(Type.TriBlockDiagonal, [3, 5, 2, 3], [3, 3, 3, 3], 32, seed=31, shift=0.05)
     elif which == "wide":
         pb = bc.random_block_problem(Type.TriBlockDiagonal, [12] * 6, [7] * 6, 16, seed=217, bounds=True, shift=0.05)
+    elif which == "n528":
+        pb = bc.random_block_problem(Type.TriBlockDiagonal, [12] * 44, [6] * 44, 4, seed=528, bounds=True, shift=0.05)
     else:
         pb, _ = bc.multiik_sequential(6, scale=1e-3)
     if s != 1.0:
@@ -359,6 +361,7 @@ FAMILY_CASES = _cases([
     ("blockgi_ref", _block("ref")),
     ("blockgi_wide", _block("wide")),
     ("blockgi_multiik", _block("multiik")),
+    ("blockgi_n528", _block("n528")),                          # eight entries of a reflector per thread (n > 512)
 ])
 
 # Part (b) / shipped-build edge tests: binade-shifted and dyadic inputs

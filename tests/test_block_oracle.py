@@ -5,7 +5,7 @@ fixtures (:172-230, :273-310; fixture solution to 1e-4, :188). CPU only."""
 import numpy as np
 import pytest
 
-from block_cases import (dense_solution, is_approx, multiik_sequential, multiik_simultaneous, po, random_block_problem)
+from block_cases import (dense_solution, dense_view, is_approx, multiik_sequential, multiik_simultaneous, po, random_block_problem)
 from jrl_qp_b200.structured import Type
 
 
@@ -107,3 +107,21 @@ def test_status_codes():
     r = po.block_solve_batch(pb.stG, pb.stC, pb.Gdata, pb.a, pb.Cdata, pb.bl, pb.bu, max_iter=1)
     full = po.block_solve_batch(pb.stG, pb.stC, pb.Gdata, pb.a, pb.Cdata, pb.bl, pb.bu)
     assert ((r["status"] == 4) == (full["iterations"] >= 1)).all()
+
+
+def test_oracle_at_n_1024_matches_kkt_reference_and_dense_solver():
+    """The oracle the GPU tests trust, at the top of the structured solver's range: [16] * 64 with bounds against the
+    extended-precision KKT solve on its active set (tests/test_warm_kkt_reference.py), the reference's testKKT and the
+    dense solver."""
+    from test_warm_kkt_reference import assert_matches_kkt_reference
+    pb = random_block_problem(Type.TriBlockDiagonal, [16] * 64, [8] * 64, 2, seed=1024, bounds=True, shift=0.05)
+    rb = _solve(pb, max_iter=1000, nthreads=2)
+    assert (rb["status"] == 0).all() and (rb["active_set"] >= 4).any()
+    flags, _, nfail = po.kkt_check_batch(rb["x"], rb["u"], pb.Gdense, pb.a, pb.Cdense, pb.bl, pb.bu, pb.xl, pb.xu, nthreads=2)
+    assert nfail == 0, flags
+    worst = assert_matches_kkt_reference(dense_view(pb), rb, sample=2, what="oracle n=1024")
+    print(f"worst error {worst:.3g} eps cond(K)")
+    rd = po.solve_batch(pb.Gdense, pb.a, pb.Cdense, pb.bl, pb.bu, pb.xl, pb.xu, max_iter=1000, nthreads=2)
+    assert np.array_equal(rb["status"], rd["status"])
+    for k in range(2):
+        assert is_approx(rb["x"][k], rd["x"][k], 1e-8) and is_approx(rb["x"][k], pb.x_planted[k], 1e-6), k

@@ -65,6 +65,9 @@ EDGE_SITES = {
 # sites of the global-workspace kernel at four rows per thread, with every proof declined
 # (initial_point_blocked runs only from the factor of a batch-shared G; a per-instance G takes the serial initial_point)
 LARGE_N_SITES = {"large_n800_cold": [(0, 1)], "large_n800_warm": [(0, 7)], "large_n800_shared": [(0, 6)]}
+# sites of the structured solver past n = 512 (blockgi_kernel<8>), with every proof declined: the small-tile factor, the
+# warp-level block solves and the blocked R solve
+BLOCKGI_N528_SITES = [(1, 10), (2, 8), (2, 9)]
 # (warm starts of the scaled problems from the unscaled cold active set: oracle parity only — the oracle itself does not
 # keep the relation there)
 RELATION_QP = ["binade_A", "binade_B", "binade_D", "binade_n70", "binade_n300"]
@@ -150,6 +153,14 @@ def test_decline_all_reaches_the_large_kernel_sites_at_n_800(variant, name):
     c = counts[name]
     missed = [f"{UNITS[u]}:{SITES[s]}" for u, s in LARGE_N_SITES[name] if c[u * NS + s] == 0]
     assert not missed, f"{name} does not reach {missed} with every proof declined (counts {_names(c)})"
+
+
+@pytest.mark.gpu
+def test_decline_all_reaches_the_blockgi_sites_above_512_variables(variant):
+    _, counts = variant["decline"]
+    c = counts["blockgi_n528"]
+    missed = [f"{UNITS[u]}:{SITES[s]}" for u, s in BLOCKGI_N528_SITES if c[u * NS + s] == 0]
+    assert not missed, f"blockgi_n528 does not reach {missed} with every proof declined (counts {_names(c)})"
 
 
 @pytest.mark.gpu

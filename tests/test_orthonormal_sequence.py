@@ -4,11 +4,16 @@ structured solver uses them — the reference's tests/InternalTest.cpp:35-323 re
     (built here with numpy from the same (essential, tau) / (c, s) data), both directions, to 1e-8, norm preserved;
   * vectors with a single non-zero segment [0; x; 0] at every position (SingleNZSegmentVector): the (start, size)
     hint of the reference only skips work on zeros, so the full application must give Q v for them;
-  * a composite sequence of four embedded transformations (InternalTest.cpp:223-323).
+  * a composite sequence of four embedded transformations (InternalTest.cpp:223-323);
+  * sequences at n = 513, 700 and 1024, where the kernel holds 5 ... 8 entries of a reflector and of the vector per thread
+    (blockgi_kernel<8>): reflectors over the whole vector and starting at the class boundaries 127 / 128, and Givens
+    records on either side of MJ * 64 rotations, the longest a thread-private stage holds (longer ones are read from
+    global memory by givens_record), up to n - 1 rotations.
 CPU part: the restatement inside oracle/block_oracle.cpp (the checker of the BlockGI kernel). GPU part (-m gpu): the
 kernel's own apply_q / apply_qt through jrlqp_blockgi_test_sequence, bit for bit against the oracle and to 1e-8
 against the dense matrix."""
 import ctypes as C
+import functools
 import os
 import sys
 
@@ -69,21 +74,18 @@ class Sequence:
 
     def householder(self, start, essential, tau):
         e = np.concatenate([[1.0], essential])
-        H = np.eye(self.n)
-        H[start:start + len(e), start:start + len(e)] -= tau * np.outer(e, e)
-        self.Q = self.Q @ H
+        cols = self.Q[:, start:start + len(e)]  # Q H = Q - tau (Q e) e^T on the columns the reflector touches
+        cols -= tau * np.outer(cols @ e, e)
         self.recs.append(("h", start, np.asarray(essential, dtype=np.float64), float(tau)))
 
     def givens(self, start, cs):
         # ElemOrthonormalSequence of Givens: G_1 G_2 ... G_k, G_i acting on (start + i, start + i + 1);
         # applyOnTheLeft(i, i+1, G): [x; y] <- [c x + s y; -s x + c y]
-        E = np.eye(self.n)
+        # Q G_i on columns a, a + 1, with G_i = [[c, s], [-s, c]] there
         for i, (c, s) in enumerate(cs):
-            G = np.eye(self.n)
             a = start + i
-            G[a, a], G[a, a + 1], G[a + 1, a], G[a + 1, a + 1] = c, s, -s, c
-            E = E @ G
-        self.Q = self.Q @ E
+            qa, qb = self.Q[:, a].copy(), self.Q[:, a + 1].copy()
+            self.Q[:, a], self.Q[:, a + 1] = c * qa - s * qb, s * qa + c * qb
         self.recs.append(("g", start, np.array([c for c, _ in cs]), np.array([s for _, s in cs])))
 
     def oracle_apply(self, v, transpose):
@@ -146,20 +148,56 @@ def _composite(rng):
 
 
 def _vectors(rng, n, seg=None):
-    """full random vectors + single-non-zero-segment vectors [0; x; 0] at every position"""
+    """full random vectors + single-non-zero-segment vectors [0; x; 0] at every position (past n = 300: at the ends and
+    across the boundaries of the 128 classes)"""
     vs = [rng.uniform(-1, 1, n)]
     ln = seg or 3
-    for i in range(n - ln + 1):
+    pos = range(n - ln + 1) if n <= 300 else sorted({p for c in range(0, n, 128) for p in (c - 2, c - 1, c, c + 1)
+                                                     if 0 <= p <= n - ln} | {n - ln})
+    for i in pos:
         v = np.zeros(n)
         v[i:i + ln] = rng.uniform(-1, 1, ln)
         vs.append(v)
     return np.array(vs)
 
 
+def _random_givens(rng, k):
+    return [make_givens(*rng.uniform(-1, 1, 2)) for _ in range(k)]
+
+
+def _large(rng, n, kind):
+    """Records of a sequence at n > 512. A thread-private stage holds the (c, s) of MJ * 64 rotations, MJ = ceil(n / 128)."""
+    seq, staged = Sequence(n), 64 * ((n + 127) // 128)
+
+    def h(start):
+        ess, tau, _ = make_householder(rng.uniform(-1, 1, n - start))
+        seq.householder(start, ess, tau)
+    if kind == "householder":
+        for start in (0, 127, 128, 500, n - 2):
+            h(start)
+    elif kind == "givens":
+        for start, k in ((130, 40), (0, staged), (n - 2 - staged, staged + 1), (0, n - 1)):
+            seq.givens(start, _random_givens(rng, k))
+    else:
+        h(0)
+        seq.givens(5, _random_givens(rng, staged + 3))
+        h(127)
+        seq.givens(120, _random_givens(rng, 50))
+        h(n - 2)
+        seq.givens(0, _random_givens(rng, n - 1))
+        h(128)
+    return seq
+
+
+@functools.lru_cache(maxsize=None)
 def _sequences():
     rng = np.random.default_rng(20261018)
-    return {"householder x3": _elem_householder(rng), "householder x1": _elem_householder(rng, k=1), "givens x5": _elem_givens(),
+    seqs = {"householder x3": _elem_householder(rng), "householder x1": _elem_householder(rng, k=1), "givens x5": _elem_givens(),
             "composite": _composite(rng), "long householder": _elem_householder(rng, n=300, k=2)}
+    for n in (513, 700, 1024):
+        for kind in ("householder", "givens", "composite"):
+            seqs[f"{kind} n={n}"] = _large(rng, n, kind)
+    return seqs
 
 
 @pytest.mark.parametrize("name", list(_sequences()))
@@ -213,3 +251,18 @@ def test_device_sequence_equals_oracle_and_dense_q(name, threads, fast, monkeypa
             assert np.abs(g - want).max() <= 1e-8 * max(1.0, np.abs(want).max())
             assert np.array_equal(g, seq.oracle_apply(v, transpose)), "kernel and oracle differ in the last bits"
     assert S.launch_count() > before
+
+
+@pytest.mark.gpu
+def test_device_sequence_refuses_more_than_1024_entries():
+    import jrl_qp_b200  # noqa: F401
+    from jrl_qp_b200 import solver as S
+    lib = S.load_library()
+    seq = Sequence(1025)
+    seq.givens(0, [make_givens(1, 2)])
+    rec, data = seq.device_records()
+    v = np.ones(1025)
+    rc = lib.jrlqp_blockgi_test_sequence(C.c_int32(0), C.c_int32(1025), C.c_int32(1), rec.ctypes.data_as(C.c_void_p),
+                                         data.ctypes.data_as(C.c_void_p), C.c_int64(len(data)), v.ctypes.data_as(C.c_void_p),
+                                         C.c_int32(1), C.c_int32(0), C.c_int32(128))
+    assert rc == -2  # JRLQP_ERR_ARG

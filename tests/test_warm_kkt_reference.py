@@ -113,7 +113,9 @@ def _sampled_instances(pb, out, sample, what):
 
 
 def assert_matches_kkt_reference(pb, out, sample=8, what=""):
-    """Up to `sample` successful instances of `out`, spread over the batch, against kkt_reference."""
+    """Up to `sample` successful instances of `out`, spread over the batch, against kkt_reference. Returns the worst error
+    of x, u and f in units of eps kappa max(1, |.|)."""
+    worst = 0.0
     for b, args in _sampled_instances(pb, out, sample, what):
         act = args[-1]
         xs, us, fs, kappa = kkt_reference(*args)
@@ -127,6 +129,10 @@ def assert_matches_kkt_reference(pb, out, sample=8, what=""):
         assert ex <= tol * max(1.0, np.abs(xs).max(initial=0.0)), f"{tag}: |x - x*| = {ex:.3g}, eps kappa = {EPS * kappa:.3g}"
         assert eu <= tol * max(1.0, np.abs(us).max(initial=0.0)), f"{tag}: |u - u*| = {eu:.3g}, eps kappa = {EPS * kappa:.3g}"
         assert abs(f - fs) <= tol * max(1.0, abs(fs)), f"{tag}: |f - f*| = {abs(f - fs):.3g}, eps kappa = {EPS * kappa:.3g}"
+        unit = EPS * kappa
+        worst = max(worst, ex / (unit * max(1.0, np.abs(xs).max(initial=0.0))), eu / (unit * max(1.0, np.abs(us).max(initial=0.0))),
+                    abs(f - fs) / (unit * max(1.0, abs(fs))))
+    return worst
 
 
 def oracle_cold(pb):
